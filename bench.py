@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the ENF steerable cross-attention hot path (forward + backward), BASELINE.json's metric.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config ns64] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config ns64] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic fields: `nef.apply` (fused cross
 attention + decode MLP) followed by the full reverse pass (latent gradients dp, da, dsigma AND all
@@ -92,6 +92,30 @@ def read_peaks():
     return dict(bf16_sustained=1400.0, bf16_burst=1590.0, hbm=6650.0, source="fallback (B200_PROFILING.md)")
 
 
+DUMP_BYTES = 64 << 20           # --dump-outputs: everything one run writes, .npy headers included
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: each named tensor -> out_dir/<name>.npy, float64 kept, every other dtype as float32, so that two builds
+    can be compared output for output.  When the tensors hold more than DUMP_BYTES together, each keeps the same fraction of its
+    elements: the flattened tensor at sorted indices drawn from a generator seeded with 0, the same sample for the same shapes."""
+    import numpy as np
+    import torch
+    arrays = {k: v.detach() for k, v in arrays.items() if v is not None}
+    size = lambda t: t.numel() * (8 if t.dtype == torch.float64 else 4)
+    keep = min(1.0, (DUMP_BYTES - 256 * len(arrays)) / max(1, sum(size(t) for t in arrays.values())))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        if keep < 1.0:
+            n = t.numel()
+            idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:int(n * keep)].sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        t = t if t.dtype == torch.float64 else t.float()
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+    print(f"bench.py: wrote {len(arrays)} arrays to {out_dir}" + (f" (a seeded sample of {keep:.3g} of each)" if keep < 1.0 else ""),
+          file=sys.stderr)
+
+
 class ClockSampler:
     """Samples SM clock / throttle reasons of one GPU during the timed region (NVML, 10 ms period)."""
 
@@ -141,6 +165,7 @@ class ClockSampler:
 # ---------------------------------------------------------------------------------------------------------
 
 def cpu_leg(cfg, steps, warmup, budget_s=25.0):
+    """budget_s: stop after this many seconds once two steps are timed (None: time all `steps`)."""
     import torch
     from oracle import enf_ref as R
     cores = os.cpu_count() or 1
@@ -178,7 +203,7 @@ def cpu_leg(cfg, steps, warmup, budget_s=25.0):
         t0 = time.perf_counter()
         step()
         times.append(time.perf_counter() - t0)
-        if time.perf_counter() - t_start > budget_s and i >= 1:
+        if budget_s is not None and time.perf_counter() - t_start > budget_s and i >= 1:
             break
     tot = sum(times)
     return dict(value=Bs * Cs * len(times) / tot, unit=UNIT, cores=cores, kind="port",
@@ -235,6 +260,7 @@ def ode_line(args):
     p_pin, a_pin, cp_pin, ca_pin = map(pin, (p_h, a_h, cp_h, ca_h))
     out_pin = torch.empty(B, Z, 2 + L).pin_memory()
     p_d, a_d, cp_d, ca_d = (t.to(dev) for t in (p_h, a_h, cp_h, ca_h))
+    last = {}           # --dump-outputs: model output and latent gradients of the latest device-resident step
 
     def step(e2e):
         if e2e:
@@ -248,6 +274,8 @@ def ode_line(args):
         ((dp * cp).sum() + (da * ca).sum()).backward()
         if e2e:
             out_pin.copy_(torch.cat([pp.grad, aa.grad], -1), non_blocking=True)
+        elif args.dump_outputs:
+            last.update(dp_dt=dp.detach(), da_dt=da.detach(), grad_p=pp.grad, grad_a=aa.grad)
 
     def timed(e2e):
         for _ in range(max(3, args.warmup)):
@@ -263,6 +291,8 @@ def ode_line(args):
 
     with ClockSampler(0) as sampler:
         ms = timed(False)
+        if args.dump_outputs:       # the end-to-end steps rebind, not overwrite, these gradients
+            outputs = {**last, **{"grad_" + k.replace("/", "."): t.grad for k, t in leaves.items()}}
         ms_e2e = timed(True)
     clocks = sampler.summary()
     n, m, F, Hd, Bd, NL, W = B * Z * Z, B * Z, ocfg.poly_dim, 128, 64, 3, 256
@@ -301,6 +331,8 @@ def ode_line(args):
             "cpu_baseline": cpu, "clocks": clocks,
             "e2e": {"value": B / (ms_e2e * 1e-3), "unit": "latent sets/s", "h2d_bytes_per_step": 4 * 2 * (p_h.numel() + a_h.numel()),
                     "d2h_bytes_per_step": 4 * out_pin.numel(), "ms_per_step": ms_e2e}}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(line))
 
 
@@ -311,6 +343,7 @@ def meta_line(args):
     all B x C queries per step; the metric counts the B x C queries once per step."""
     import torch
     import enf_pde_b200 as E
+    from enf_pde_b200 import _lib
     cfg = dict(CONFIGS[args.config])
     assert torch.cuda.is_available(), "bench.py --meta needs a CUDA device"
     dev = torch.device("cuda", 0)
@@ -332,12 +365,15 @@ def meta_line(args):
     masks = [torch.arange(C, device=dev) for _ in range(K + 1)]       # every query at every step (the reference sub-samples to fit memory)
     p_d, a_d = p_h.to(dev), a_h.to(dev)
     s_d = s_h.to(dev) if cfg["window"] else None
+    last = {}           # --dump-outputs: loss and adapted latents of the latest step
 
     def step():
         for t in leaves:
             t.grad = None
-        loss, _ = E.inner_loop(nef, variables, x_d, img, p_d, a_d, s_d, lrs, K, masks=masks)
+        loss, adapted = E.inner_loop(nef, variables, x_d, img, p_d, a_d, s_d, lrs, K, masks=masks)
         loss.backward()
+        if args.dump_outputs:
+            last.update({"loss": loss.detach(), **{"adapted_" + k: t.detach() for k, t in zip(("p", "a", "gaussian_window"), adapted) if t is not None}})
         return loss
 
     for _ in range(max(3, args.warmup)):
@@ -355,6 +391,8 @@ def meta_line(args):
     flop = (K + 1) * 3.0 * (f_alg * B * C * Z + flops_per_query_tail(cfg) * B * C)
     peaks = read_peaks()
     ach = flop / (ms * 1e-3) / 1e12
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {**last, **{"grad_" + n: t.grad for n, t in zip(_lib.LEAVES, leaves) if t is not None}})
     print(json.dumps({"metric": "coord-queries/sec (first-order Meta-SGD training step: 3 inner steps + outer fwd+bwd)", "value": B * C / (ms * 1e-3),
                       "unit": "queries/s", "n_gpus": 1, "steps": args.steps, "warmup": max(3, args.warmup), "ms_per_step": ms,
                       "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f16 operands / f32 accumulate (tcgen05) + f32",
@@ -397,7 +435,14 @@ def main():
                     help="first-order Meta-SGD training step line (SURVEY 8f-1): K = 3 latents-only inner steps + the outer fwd+bwd")
     ap.add_argument("--ode", action="store_true",
                     help="latent ODE model line (SURVEY 8f-3): PonitaODEGen fwd + bwd at config_navier_stokes.yaml's `node:` sizes")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last device-resident step returned (output, loss, gradients) as "
+                         "DIR/<name>.npy, float32 (float64 kept), at most 64 MB in all (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
     if args.ode:
         return ode_line(args)
     if args.meta:
@@ -418,7 +463,7 @@ def main():
         kind, why = reference_probe()
         workload = {"workload": f"{args.config}: {cfg['label']}", "B_per_gpu": cfg["B"], "C": C_full, "Z": cfg["Z"], "d": cfg["d"],
                     "H": cfg["H"], "invariant": cfg["invariant_type"], "latent_dim": cfg["L"], "num_out": cfg["O"]}
-        r = cpu_leg(cfg, max(1, args.steps), args.warmup, budget_s=120.0)
+        r = cpu_leg(cfg, args.steps, args.warmup, budget_s=None)
         line = {"impl": "reference", "metric": METRIC, "value": r["value"], "unit": UNIT, "n_gpus": args.gpus,
                 "steps": r["steps"], "warmup": args.warmup, "ms_per_step": r["ms_per_step"], "higher_is_better": True,
                 "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic", "config": workload,
@@ -480,11 +525,14 @@ def main():
     x_d, y_d = x_h.to(dev), y_h.to(dev)
     p_d, a_d, s_d = (t.to(dev).requires_grad_(not args.forward_only) for t in (p_h, a_h, s_h))
     n_out = B_global * C_full * cfg["O"] if args.scaling == "strong" else B * C * cfg["O"]
+    last = {}           # --dump-outputs: decoded field (detached: its graph holds the workspace) and loss of the latest step
 
     def step_device(x, y, p, a, s):
         if args.forward_only:
             with torch.no_grad():
                 out = nef.apply(variables, x[None].expand(B, -1, -1), p, a, s if use_sigma else None)
+            if args.dump_outputs:
+                last["out"] = out
             return out
         for t in leaves:
             t.grad = None
@@ -494,6 +542,8 @@ def main():
         out = nef.apply(variables, x[None].expand(B, -1, -1), p, a, s if use_sigma else None)
         diff = out.detach() - y
         loss = (diff * diff).mean()
+        if args.dump_outputs:
+            last.update(out=out.detach(), loss=loss)
         out.backward(diff * (2.0 / n_out))
         if world > 1:
             if partition == "queries":      # latent gradients are sums over queries too: one packed collective for both
@@ -523,6 +573,11 @@ def main():
         ev1.record()
         barrier()
     ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs:       # what the last timed step handed its caller; the end-to-end steps below rebind, not overwrite, these
+        outputs = dict(last)
+        if not args.forward_only:
+            outputs.update(grad_p=p_d.grad, grad_a=a_d.grad, grad_gaussian_window=s_d.grad if use_sigma else None)
+            outputs.update({"grad_" + n: t.grad for n, t in zip(_lib.LEAVES, leaves) if t is not None})
     buf = (ctypes.c_float * 256)()
     n_f = lib.enf_profile_collect(0, buf, 256); fwd_ms = [buf[i] for i in range(max(n_f, 0))]
     n_b = lib.enf_profile_collect(1, buf, 256); bwd_ms = [buf[i] for i in range(max(n_b, 0))]
@@ -673,6 +728,8 @@ def main():
             "e2e": {"value": q_total / (ms_e2e * 1e-3), "unit": UNIT, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
                     "ms_per_step": ms_e2e / args.steps},
             "gpu_launches": launches}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
