@@ -8,7 +8,6 @@
 // and the reverse of each for enf_xattn_bwd.  The algebra is tests/folded_model.py (validated on CPU
 // against the unfused oracle); DESIGN.md lists every buffer.
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <map>
 #include <mutex>
@@ -145,7 +144,6 @@ Layout make_layout(const EnfDesc& D, const EnfRecordLayout& rl) {
     const size_t dimg = d * (d < 64 ? 64 : d) / 2;
     Y.add("img_q_w1", dimg); Y.add("img_v_w1", dimg); Y.add("img_Wp", dimg); Y.add("img_W3", BZ * H * dimg);
     if (train) Y.add("slog", BC * (size_t)D.Z * H);
-    Y.add("dbg_fwd", 8192);
     // tf32 stage GEMMs: activated copies of the decode-MLP pre-activations (their A operands arrive by TMA) and the
     // low parts W - trunc_tf32(W) of the weights those GEMMs multiply by (3-term split product)
     Y.add("fo_act", BC * Hd); Y.add("o1_act", BC * d); Y.add("o2_act", BC * d);
@@ -159,7 +157,6 @@ Layout make_layout(const EnfDesc& D, const EnfRecordLayout& rl) {
       Y.add("dthat", cZ * Cpad * d / 2); Y.add("ds_tc", cC * (size_t)D.Z * H); Y.add("Dg", BC * H);
       Y.add("dnb16", (size_t)D.B * Cpad * Hd / 2);
       Y.add("duv", cC * (size_t)D.Z * 8);
-      Y.add("dbg", 8192);
       // fp16 operand images of `that` per (field, latent, 128-query tile), stashed by the forward for backward kernel A
       Y.add("that_img", cZ * Cpad * (d < 64 ? 64 : d) / 2);
       // rstd * gelu' of the same layer (fp16), stashed for backward kernel B: with `that` it is all the LayerNorm / gelu backward needs
@@ -553,8 +550,6 @@ int enf_xattn_fwd(const EnfDesc* desc, const EnfWeights* w, const float* x, int6
     // ENF_FLAG_RECOMPUTE: no per-pair operand stash now; the backward rebuilds it chunk by chunk
     const bool stash = train && use_tc_bwd(D) && !(D.flags & ENF_FLAG_RECOMPUTE);
     EnfPairTcParams tp = tc_fwd_params(D, rl, *w, c, pp, train, stash);
-    static const bool trace_fwd = getenv("ENF_DEBUG_TRACE") != nullptr;
-    tp.dbg = trace_fwd ? reinterpret_cast<long long*>(c.f("dbg_fwd")) : nullptr;
     prof_mark(0, 0, st);
     nl = enf_launch_pairs_fwd_tc(st, d, H, tp);
     prof_mark(0, 1, st);
@@ -742,9 +737,6 @@ int enf_xattn_bwd(const EnfDesc* desc, const EnfWeights* w, const float* x, int6
     tp.dnbar = c.f("s0"); tp.Dg = c.f("Dg"); tp.gmax = c.f("gmax"); tp.dnb16 = reinterpret_cast<uint4*>(c.f("dnb16"));
     tp.that_img = reinterpret_cast<const uint8_t*>(c.f("that_img"));
     tp.dgr = reinterpret_cast<const uint4*>(c.f("dgr")); tp.trstd = c.f("trstd");
-    static const bool trace = getenv("ENF_DEBUG_TRACE") != nullptr;
-    tp.dbg = trace ? reinterpret_cast<long long*>(c.f("dbg")) : nullptr;
-    { const char* e = getenv("ENF_DEBUG_NOSPLIT"); tp.debug_nosplit = (e && e[0] == '1') ? 1 : 0; }
     tp.dthat = reinterpret_cast<__half*>(c.f("dthat")); tp.ds = c.f("ds_tc"); tp.duv = c.f("duv");
     tp.g_W3 = c.f("g_W3"); tp.g_b3 = c.f("g_b3");
     if (wg) {        // latents-only backward: kernels B / C skip the shared-weight gradient MMAs and their flush

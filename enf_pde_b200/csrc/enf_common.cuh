@@ -192,7 +192,6 @@ struct EnfPairTcParams {
   uint4* dgr;                                // gelu'(tpre) of the same layer, fp16, in backward kernel B's load order (the chunked
                                              // order of dthat below); stashed together with that_img, null when that is
   float* trstd;                              // [B,Z,ceil(C/128)*128] reciprocal standard deviation of that LayerNorm (with dgr)
-  long long* dbg;                            // optional clock64() trace of one CTA (diagnostics; null in production)
 };
 bool enf_pairs_fwd_tc_supported(int d, int H);
 int enf_launch_pairs_fwd_tc(cudaStream_t st, int d, int H, const EnfPairTcParams& p);
@@ -224,8 +223,6 @@ struct EnfPairTcBwdParams {
   float* g_W3; float* g_b3;                  // per-latent outputs of A
   float* g_q_w1; float* g_q_b1; float* g_v_w1; float* g_v_b1; float* g_Wp; float* g_bp;   // shared-weight grads (atomics)
   float* g_U; float* g_kappa; float* g_lam; float* g_sigma;                                // per-latent outputs of B
-  long long* dbg;                            // optional clock64() trace of one CTA (diagnostics; null in production)
-  int debug_nosplit;                         // diagnostics (ENF_DEBUG_NOSPLIT): kernels B / C drop the low terms of their relu GEMMs
 };
 bool enf_pairs_bwd_tc_supported(int d, int H);
 // prep (once per backward, whole batch): gradient scale, fp16 cotangent of nbar, Dg;  main: kernels A, B, C on p.B fields

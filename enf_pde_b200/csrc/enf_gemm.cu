@@ -3,8 +3,6 @@
 // this kernel favours generality (arbitrary strides => transposes and head-sliced views for free)
 // over peak throughput.  64x64x16 tiles, 256 threads, 4x4 register tile per thread, 8-stage cp.async pipeline
 // (most calls are tiny fold / unfold products whose time is global-load latency, not flops).
-#include <cstdlib>
-
 #include "enf_common.cuh"
 
 namespace {
@@ -196,8 +194,7 @@ int enf_gemm_group(cudaStream_t st, int n, const EnfGemmProblem* p) {
 
 int enf_gemm(cudaStream_t st, int M, int N, int K, EnfMat A, EnfMat B, EnfMat C, const EnfGemmOpts& o) {
   if (M <= 0 || N <= 0 || o.batch <= 0) return 0;
-  static const bool no_tc = getenv("ENF_DEBUG_NO_TC_GEMM") != nullptr;     // A/B switch for numerics debugging
-  if (o.tc && !no_tc) {
+  if (o.tc) {
     int r = enf_gemm_tc(st, M, N, K, A, B, C, o);
     if (r != 0) return r;
   }

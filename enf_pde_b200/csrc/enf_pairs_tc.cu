@@ -61,14 +61,6 @@ template <int D, int H> struct TcCfg {
   static_assert(SMEM_BYTES <= 227 * 1024, "shared memory budget");
 };
 
-// diagnostics (build with `make TRACE=1`, run with ENF_DEBUG_TRACE=1): clock64() of selected events of CTA (7, 0),
-// latents 8..11, thread 32
-#ifdef ENF_TRACE
-#define F_STAMP(slot) do { if (P.dbg && blockIdx.x == 7 && blockIdx.y == 0 && tid == 32 && z >= 8 && z < 12) P.dbg[(z - 8) * 32 + (slot)] = clock64(); } while (0)
-#else
-#define F_STAMP(slot) do { } while (0)
-#endif
-
 template <int D, int H>
 __global__ void __launch_bounds__(TcCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_fwd_tc_kernel(EnfPairTcParams P) {
   using C = TcCfg<D, H>;
@@ -213,7 +205,6 @@ __global__ void __launch_bounds__(TcCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_fwd_tc
     const uint32_t par = z & 1;
     const int64_t bz = (int64_t)b * P.Z + z;
     const bool more = z + 1 < P.Z;
-    F_STAMP(0);
     // ---- (a) RFF phases of this latent (its invariants were written during the previous latent's E4); prefetch of the
     //          next latent's vectors; gamma_q, gamma_v from the phases
     if (more) prefetch_latent(z + 1);
@@ -223,7 +214,6 @@ __global__ void __launch_bounds__(TcCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_fwd_tc
     const float* s_kap = s_b3 + H * D;
     tc::mbar_wait(bar_p, par);
     tc::tc_fence_after();
-    F_STAMP(1);
     // gamma_q first: GEMM1 is issued as soon as its operand is complete (named barrier 7: warp 0 syncs, the others arrive)
     // and runs in the shadow of the gamma_v pass
     rff_from_proj<D, false>(tp + lane_off + 16 * cq, sA0, nullptr, C::ABLK, row, 16 * cq);
@@ -241,11 +231,9 @@ __global__ void __launch_bounds__(TcCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_fwd_tc
       tc::named_arrive(7, C::NT);
     }
     rff_from_proj<D, false>(tp + lane_off + HD + 16 * cq, sA1, nullptr, C::ABLK, row, 16 * cq);
-    F_STAMP(2);
     tc::tc_fence_before();
     tc::fence_proxy_async();
     __syncthreads();
-    F_STAMP(3);
     if (tid == 0) {
       tc::tc_fence_after();
       issue_gemm<D>(t0, aA1, aW + C::WIMG, C::ABLK, C::WBLK);
@@ -254,10 +242,8 @@ __global__ void __launch_bounds__(TcCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_fwd_tc
     const float win = s_win[par * ROWS + row];
     // ---- (c) E1: h1q = relu(T0 + b1q); logit partials (overlaps GEMM2) -------------------------------------
     float v[32];
-    F_STAMP(4);
     tc::mbar_wait(bar_g1, par);
     tc::tc_fence_after();
-    F_STAMP(5);
     tc::tmem_ld32(t1 + my_t, v);
     tc::tmem_ld_wait();
     {
@@ -280,10 +266,8 @@ __global__ void __launch_bounds__(TcCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_fwd_tc
       for (int h = 0; h < H; ++h) s_spart[(cq * ROWS + row) * H + h] = part[h].x + part[h].y;
     }
     // ---- (d) E2: h1v = relu(T1 + b1v) -> A0 ----------------------------------------------------------------
-    F_STAMP(6);
     tc::mbar_wait(bar_g2, par);
     tc::tc_fence_after();
-    F_STAMP(7);
     tc::tmem_ld32(t0 + my_t, v);
     tc::tmem_ld_wait();
 #pragma unroll
@@ -299,11 +283,9 @@ __global__ void __launch_bounds__(TcCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_fwd_tc
       }
       tc::st_row8_bf16(sA0, C::ABLK, row, col0 + c8, o);
     }
-    F_STAMP(8);
     tc::tc_fence_before();
     tc::fence_proxy_async();
     __syncthreads();
-    F_STAMP(9);
     if (tid == 0) {
       tc::tc_fence_after();
       issue_gemm<D>(t0, aA0, aW + 2 * C::WIMG, C::ABLK, C::WBLK);
@@ -326,10 +308,8 @@ __global__ void __launch_bounds__(TcCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_fwd_tc
     }
     uint32_t dgh[16];                          // my 32 columns of the backward's stash gelu'(tpre) (fp16), parked E3 -> E4_0
     // ---- (e) E3: g = gelu(T0 + b'), row statistics, LayerNorm -> A1 ----
-    F_STAMP(10);
     tc::mbar_wait(bar_g3, par);
     tc::tc_fence_after();
-    F_STAMP(11);
     if (H > 1 && !C::kStageAll && tid == 0) {          // A0 is free again: stream W3[z,1] into it
       tc::mbar_expect_tx(&bar_w3[1], C::WIMG);
       tc::bulk_g2s(sA0, P.img_W3 + (bz * H + 1) * C::WIMG, C::WIMG, &bar_w3[1]);
@@ -340,10 +320,8 @@ __global__ void __launch_bounds__(TcCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_fwd_tc
       float st[2];
       if (P.dgr) gelu_rowsums32_stash(v, s_bias + 2 * D + col0, dgh, st);      // + gelu' of this layer, packed, for the backward
       else gelu_rowsums32(v, s_bias + 2 * D + col0, st);
-      F_STAMP(12);
       xw = 0;
       row_exchange<C::NQ, 2>(s_exch, xw, cq, row, lq, st);
-      F_STAMP(13);
       const float mu = st[0] * (1.f / D);
       const float rstd = rsqrtf(fmaxf(st[1] * (1.f / D) - mu * mu, 0.f) + 1e-6f);
       const float2 rstd2 = tc::splat2(rstd), nm2 = tc::splat2(-mu * rstd);
@@ -356,12 +334,10 @@ __global__ void __launch_bounds__(TcCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_fwd_tc
       }
       if (P.dgr && cq == 0) P.trstd[(size_t)bz * gridDim.x * ROWS + c0 + row] = rstd;
     }
-    F_STAMP(14);
     tc::cp_async_wait_all();                  // the next latent's vectors (requested at the top) are visible after this barrier
     tc::tc_fence_before();
     tc::fence_proxy_async();
     __syncthreads();
-    F_STAMP(15);
     if (tid == 0) {
       if (P.that_img) {                // stash the that operand tile for backward kernel A (bulk store, no thread work)
         tc::bulk_s2g(P.that_img + ((size_t)bz * gridDim.x + blockIdx.x) * C::ATILE, sA1, C::ATILE);
@@ -388,7 +364,6 @@ __global__ void __launch_bounds__(TcCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_fwd_tc
     for (int h = 0; h < H; ++h) {
       tc::mbar_wait(&bar_g4[h], par);
       tc::tc_fence_after();
-      F_STAMP(16 + 2 * h);
       tc::tmem_ld32(((h & 1) ? t1 : t0) + my_t, v);
       tc::tmem_ld_wait();
       if (h == 0 && (more || P.dgr || H == 3)) {
@@ -439,7 +414,6 @@ __global__ void __launch_bounds__(TcCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_fwd_tc
 #pragma unroll
       for (int j = 0; j < 32; j += 2) tc::st2(a + j, tc::fma2(tc::ld2(v + j), pr2, tc::fma2(tc::ld2(a + j), corr2, tz2)));
       tc::tmem_st32(tacc + h * D + my_t, a);
-      F_STAMP(17 + 2 * h);
     }
     if (tid == 0) {
       if (P.that_img) tc::bulk_wait_read0();   // the stashes have been read out of A1 / the stage buffer before they are overwritten
@@ -451,7 +425,6 @@ __global__ void __launch_bounds__(TcCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_fwd_tc
     tc::tmem_st_wait();
     tc::tc_fence_before();
     __syncthreads();
-    F_STAMP(20);
   }
 
 #pragma unroll

@@ -120,29 +120,19 @@ template <int D, int H> struct ACfg {
   static_assert(SMEM_BYTES <= 227 * 1024, "shared memory budget");
 };
 
-// Warp roles: warps 0..15 are the epilogue warps (thread layout of enf_pairs_tc_common.cuh); warp 16 only issues --
-// bulk copies, tcgen05.mma, commits.  Epilogue warps never block on each other: when their part of an operand tile is
-// written they ARRIVE on a named barrier the issue warp SYNCs on, and go on with whatever does not need that MMA.
+// Warp roles: all 16 warps run the epilogues (thread layout of enf_pairs_tc_common.cuh) and never block on each other:
+// when their part of an operand tile is written they ARRIVE on a named barrier the issuing warp SYNCs on, and go on with
+// whatever does not need that MMA.
 constexpr int kABarHead = 5;      // + h (h < 3): dm_h tile written              (named barriers 1..4 belong to row_exchange)
 constexpr int kABarDth = 8;       // dthat of the tile has been read out of TMEM
 using tc::named_arrive;
 using tc::named_sync;
 
-// diagnostics (build with `make TRACE=1`, run with ENF_DEBUG_TRACE=1): clock64() of selected events of CTA 7, tiles 4..7,
-// for thread `who`
-#ifdef ENF_TRACE
-#define A_STAMP(who, slot) do { if (P.dbg && blockIdx.x == 7 && tid == (who) && ct >= 4 && ct < 8) P.dbg[((who) == 512 ? 512 : 0) + (ct - 4) * 32 + (slot)] = clock64(); } while (0)
-#else
-#define A_STAMP(who, slot) do { } while (0)
-#endif
-
-// SEP = true: a 17th warp issues (96 registers per thread: the register file is granted in units of 4 warps);
-// SEP = false: warp 0 issues between its own epilogue phases (it SYNCs on the named barriers, the others ARRIVE), 128 registers.
-template <int D, int H, bool SEP>
-__global__ void __launch_bounds__(BwdCfg<D, H>::NT + (SEP ? 32 : 0), D <= 64 ? 2 : 1) pairs_bwd_tc_a_kernel(EnfPairTcBwdParams P) {
+// Warp 0 issues (bulk copies, tcgen05.mma, commits) between its own epilogue phases.
+template <int D, int H>
+__global__ void __launch_bounds__(BwdCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_bwd_tc_a_kernel(EnfPairTcBwdParams P) {
   using C = BwdCfg<D, H>;
   using A = ACfg<D, H>;
-  constexpr int NTA = C::NT + (SEP ? 32 : 0);         // epilogue threads (+ the issue warp)
   extern __shared__ uint8_t smem_raw[];
   uint8_t* base = smem_raw + ((1024u - (tc::smem_u32(smem_raw) & 1023u)) & 1023u);   // 1024-aligned; pointer stays in the shared address space (LDS/STS, not generic LD/ST)
   uint8_t* sW3 = base + A::OFF_W3;
@@ -158,7 +148,6 @@ __global__ void __launch_bounds__(BwdCfg<D, H>::NT + (SEP ? 32 : 0), D <= 64 ? 2
   uint32_t* s_tmem = reinterpret_cast<uint32_t*>(bars + 8);
 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const bool issuer = SEP && warp == 16;
   const int lq = warp & 3, cq = warp >> 2;
   const int row = lq * 32 + lane, col0 = cq * 32;
   const int64_t bz = blockIdx.x;
@@ -177,7 +166,7 @@ __global__ void __launch_bounds__(BwdCfg<D, H>::NT + (SEP ? 32 : 0), D <= 64 ? 2
   constexpr int kTmemNeed = (kWork + H) * D;
   constexpr int kTmemCols = kTmemNeed <= 128 ? 128 : kTmemNeed <= 256 ? 256 : 512;
   if (warp == 0) tc::tmem_alloc<kTmemCols>(s_tmem);
-  for (int e = tid; e < H * D; e += NTA) { s_b3[e] = P.b3[bz * H * D + e]; s_db3[e] = 0.f; }
+  for (int e = tid; e < H * D; e += C::NT) { s_b3[e] = P.b3[bz * H * D + e]; s_db3[e] = 0.f; }
   float gs, inv_gs;
   load_scale(P.gmax, gs, inv_gs);
   tc::tc_fence_before();
@@ -241,209 +230,175 @@ __global__ void __launch_bounds__(BwdCfg<D, H>::NT + (SEP ? 32 : 0), D <= 64 ? 2
     }
   };
 
-  if (issuer) {
-    // ================================ issue warp =================================================================
-    const bool lead = tc::elect_one();
-    if (lead) issue_prologue();
-    for (int ct = 0; ct < ntiles; ++ct) {
-      if (ct > 0) named_sync(kABarDth, NTA);
-      if (lead) issue_top(ct);
+  int xw = 0;
+  // per-row scalars of tile `ct` (logits, log-sum-exp, Dg of my row, all heads) -> shared, without passing through registers
+  auto prefetch_rows = [&](int ct) {
+    const int c = ct * ROWS + row;
+    if (cq == 0 && c < P.C) {
+      const int64_t q = (int64_t)b * P.C + c;
+      float* dst = s_rs + (ct & 1) * 3 * ROWS * H + row * H;
+      if (H == 3) {        // 12 bytes is not a cp.async size
 #pragma unroll
-      for (int h = 0; h < H; ++h) {
-        named_sync(kABarHead + h, NTA);
-        if (lead) issue_head(ct, h);
-        __syncwarp();
+        for (int h = 0; h < H; ++h) {
+          tc::cp_async<4>(dst + h, P.slog + (bz * P.C + c) * H + h);
+          tc::cp_async<4>(dst + ROWS * H + h, P.lse + q * H + h);
+          tc::cp_async<4>(dst + 2 * ROWS * H + h, P.Dg + q * H + h);
+        }
+      } else {
+        constexpr int kB = 4 * (H == 3 ? 1 : H);
+        tc::cp_async<kB>(dst, P.slog + (bz * P.C + c) * H);
+        tc::cp_async<kB>(dst + ROWS * H, P.lse + q * H);
+        tc::cp_async<kB>(dst + 2 * ROWS * H, P.Dg + q * H);
       }
     }
-  } else {
-    // ================================ epilogue warps ==============================================================
-    int xw = 0;
-    // per-row scalars of tile `ct` (logits, log-sum-exp, Dg of my row, all heads) -> shared, without passing through registers
-    auto prefetch_rows = [&](int ct) {
-      const int c = ct * ROWS + row;
-      if (cq == 0 && c < P.C) {
-        const int64_t q = (int64_t)b * P.C + c;
-        float* dst = s_rs + (ct & 1) * 3 * ROWS * H + row * H;
-        if (H == 3) {        // 12 bytes is not a cp.async size
+  };
+  if (warp == 0) {
+    if (tc::elect_one()) issue_prologue();
+    __syncwarp();
+  }
+  prefetch_rows(0);
+  uint4 dnq[4];                                      // my 32 columns of the scaled fp16 cotangent of nbar, (tile, head) about to be processed
+  auto load_dnb = [&](int ct, int h) {
+    const uint4* src = P.dnb16 + ((((int64_t)b * ntiles + ct) * H + h) * C::NQ + cq) * 4 * ROWS + row;
 #pragma unroll
-          for (int h = 0; h < H; ++h) {
-            tc::cp_async<4>(dst + h, P.slog + (bz * P.C + c) * H + h);
-            tc::cp_async<4>(dst + ROWS * H + h, P.lse + q * H + h);
-            tc::cp_async<4>(dst + 2 * ROWS * H + h, P.Dg + q * H + h);
-          }
-        } else {
-          constexpr int kB = 4 * (H == 3 ? 1 : H);
-          tc::cp_async<kB>(dst, P.slog + (bz * P.C + c) * H);
-          tc::cp_async<kB>(dst + ROWS * H, P.lse + q * H);
-          tc::cp_async<kB>(dst + 2 * ROWS * H, P.Dg + q * H);
-        }
-      }
-    };
-    if (!SEP && warp == 0) {
-      if (tc::elect_one()) issue_prologue();
+    for (int q = 0; q < 4; ++q) dnq[q] = __ldg(src + q * ROWS);       // a warp reads 512 contiguous bytes per instruction
+  };
+  load_dnb(0, 0);
+
+  for (int ct = 0; ct < ntiles; ++ct) {
+    const uint32_t par = ct & 1;
+    const int e = ct & 1;                            // region roles of this tile: first = region e, other = region e ^ 1
+    const uint32_t tF = tm + e * D, tS = tm + (e ^ 1) * D;
+    const int c0 = ct * ROWS;
+    const bool valid = c0 + row < P.C;
+    if (warp == 0) {                                 // warp 0 doubles as the issuer
+      if (ct > 0) named_sync(kABarDth, C::NT);
+      if (tc::elect_one()) issue_top(ct);
       __syncwarp();
     }
-    prefetch_rows(0);
-    uint4 dnq[4];                                      // my 32 columns of the scaled fp16 cotangent of nbar, (tile, head) about to be processed
-    auto load_dnb = [&](int ct, int h) {
-      const uint4* src = P.dnb16 + ((((int64_t)b * ntiles + ct) * H + h) * C::NQ + cq) * 4 * ROWS + row;
+    tc::cp_async_wait_all();                         // this tile's row scalars (issued a tile ago by the cq == 0 thread of the row);
+                                                     // the row's other threads read them after the row_exchange barrier below
+    if (ct + 1 < ntiles) prefetch_rows(ct + 1);
+    float v[32];
 #pragma unroll
-      for (int q = 0; q < 4; ++q) dnq[q] = __ldg(src + q * ROWS);       // a warp reads 512 contiguous bytes per instruction
-    };
-    load_dnb(0, 0);
-
-    for (int ct = 0; ct < ntiles; ++ct) {
-      const uint32_t par = ct & 1;
-      const int e = ct & 1;                            // region roles of this tile: first = region e, other = region e ^ 1
-      const uint32_t tF = tm + e * D, tS = tm + (e ^ 1) * D;
-      const int c0 = ct * ROWS;
-      const bool valid = c0 + row < P.C;
-      if (!SEP && warp == 0) {                         // warp 0 doubles as the issuer
-        if (ct > 0) named_sync(kABarDth, NTA);
-        if (tc::elect_one()) issue_top(ct);
-        __syncwarp();
-      }
-      A_STAMP(32, 0);
-      tc::cp_async_wait_all();                         // this tile's row scalars (issued a tile ago by the cq == 0 thread of the row);
-                                                       // the row's other threads read them after the row_exchange barrier below
-      if (ct + 1 < ntiles) prefetch_rows(ct + 1);
-      float v[32];
-      A_STAMP(32, 1);
-#pragma unroll
-      for (int h = 0; h < H; ++h) {
-        tc::mbar_wait(&bar_g4[h], par);
-        tc::tc_fence_after();
-        A_STAMP(32, 2 + 8 * h);
-        tc::tmem_ld32((h == 0 ? tF : h == 1 ? tS : tR2) + my_t, v);
-        tc::tmem_ld_wait();
-        A_STAMP(32, 3 + 8 * h);
-        // one pass, one exchange: with g = gelu(m), n = (g - mu) rstd the row sums the LayerNorm backward needs are
-        //   sum_j dnb_j n_j = rstd (sum dnb g - mu sum dnb)   and   sum_j dnb_j
-        uint32_t dgh[16];                              // gelu', packed to fp16 inside the pass (dm is rounded to fp16 for the MMAs anyway)
-        uint32_t gh[16];                               // g, packed to fp16 once the row sums have seen it in fp32 (it only re-enters
-                                                       // through the small LayerNorm projection term of dm): 16 registers instead of 32
-        float st[4];
-        {
-          float st01[2];
-          gelu_rowsums32_stash(v, s_b3 + h * D + col0, dgh, st01);
-          st[0] = st01[0]; st[1] = st01[1];
-        }
-        // the cotangent rows were requested one phase ago; touching them only now keeps their L2 latency off the gelu pass
-        {
-          float2 s2 = tc::splat2(0.f), s3 = tc::splat2(0.f);
-#pragma unroll
-          for (int j4 = 0; j4 < 32; j4 += 4) {
-            const __half2* h2 = reinterpret_cast<const __half2*>(&dnq[j4 >> 3]) + ((j4 & 4) >> 1);     // dnb[j4 .. j4 + 3], packed
-            const float2 d01 = __half22float2(h2[0]), d23 = __half22float2(h2[1]);
-            s2 = tc::fma2(d01, tc::ld2(v + j4), s2); s3 = tc::add2(s3, d01);
-            s2 = tc::fma2(d23, tc::ld2(v + j4 + 2), s2); s3 = tc::add2(s3, d23);
-            gh[j4 >> 1] = tc::pack_bf16(v[j4], v[j4 + 1]);
-            gh[(j4 >> 1) + 1] = tc::pack_bf16(v[j4 + 2], v[j4 + 3]);
-          }
-          st[2] = s2.x + s2.y; st[3] = s3.x + s3.y;
-        }
-        A_STAMP(32, 4 + 8 * h);
-        row_exchange<C::NQ, 4>(s_exch, xw, cq, row, lq, st);
-        A_STAMP(32, 5 + 8 * h);
-        float att = 0.f, Dh = 0.f;
-        if (valid) {
-          const float* rs = s_rs + e * 3 * ROWS * H + row * H + h;
-          att = __expf(rs[0] - rs[ROWS * H]);
-          Dh = rs[2 * ROWS * H];
-        }
-        const float atts = att;                        // dnb16 already carries the scale gs
-        const float mu = st[0] * (1.f / D);
-        const float rstd = rsqrtf(fmaxf(st[1] * (1.f / D) - mu * mu, 0.f) + 1e-6f);
-        const float dd0 = rstd * (st[2] - mu * st[3]), dd1 = st[3];
-        const float dsh = atts * (dd0 - Dh * gs);
-        const float mean1 = atts * dd1 * (1.f / D), mean2 = atts * dd0 * (1.f / D);
-        // dm = rstd (att dnb - mean1 - n mean2) g'   with n = (g - mu) rstd, constants folded
-        const float ka = atts * rstd, kc = rstd * (mu * rstd * mean2 - mean1), kb = rstd * rstd * mean2;
-        uint8_t* sDh = sDm + h * C::ATILE;
-        if (h == 0 && ct > 0) tc::mbar_wait(bar_gb, par ^ 1);      // every MMA of the previous tile is done with the dm tiles
-#pragma unroll
-        uint32_t dmh[16];                              // dm as the fp16 operand words the MMAs read; the bias column sums add the same words
-#pragma unroll
-        for (int c8 = 0; c8 < 32; c8 += 8) {
-          const __half2* h2 = reinterpret_cast<const __half2*>(&dnq[c8 >> 3]);
-          const __half2* g2 = reinterpret_cast<const __half2*>(&gh[c8 >> 1]);
-          const __half2* d2 = reinterpret_cast<const __half2*>(&dgh[c8 >> 1]);
-#pragma unroll
-          for (int t = 0; t < 4; ++t) {
-            const float2 dv = __half22float2(h2[t]), gv = __half22float2(g2[t]);
-            const float2 dm = tc::mul2(tc::fma2(gv, tc::splat2(-kb), tc::fma2(tc::splat2(ka), dv, tc::splat2(kc))), __half22float2(d2[t]));
-            dmh[(c8 >> 1) + t] = tc::pack_bf16(dm.x, dm.y);
-          }
-          tc::st_row8_words(sDh, C::ABLK, row, col0 + c8, dmh + (c8 >> 1));
-        }
-        A_STAMP(32, 21 + 3 * h);
-        tc::fence_proxy_async();
-        A_STAMP(32, 22 + 3 * h);
-        tc::tc_fence_before();
-        if (!SEP && warp == 0) {
-          named_sync(kABarHead + h, NTA);
-          if (tc::elect_one()) issue_head(ct, h);
-          __syncwarp();
-        } else {
-          named_arrive(kABarHead + h, NTA);            // the issuer takes it from here
-        }
-        A_STAMP(32, 6 + 8 * h);
-        // fetch the cotangent rows of the next (tile, head) now, a whole phase ahead of their use
-        if (h + 1 < H) load_dnb(ct, h + 1);
-        else if (ct + 1 < ntiles) load_dnb(ct + 1, 0);
-        {
-          float cs = warp_colsum32_h2(dmh, lane);
-          A_STAMP(32, 23 + 3 * h);
-          atomicAdd(&s_db3[h * D + col0 + lane], cs);
-        }
-        if (cq == 0 && valid) P.ds[((bz * P.C) + c0 + row) * H + h] = dsh;
-        A_STAMP(32, 7 + 8 * h);
-      }
-      // dthat = sum_h dm_h W3_h^T -> global (fp16, scaled)
-      tc::mbar_wait(bar_d, par);
+    for (int h = 0; h < H; ++h) {
+      tc::mbar_wait(&bar_g4[h], par);
       tc::tc_fence_after();
-      A_STAMP(32, 18);
-      tc::tmem_ld32(tF + my_t, v);
+      tc::tmem_ld32((h == 0 ? tF : h == 1 ? tS : tR2) + my_t, v);
       tc::tmem_ld_wait();
-      A_STAMP(32, 19);
-      tc::tc_fence_before();
-      if (ct + 1 < ntiles && (SEP || warp != 0)) named_arrive(kABarDth, NTA);     // tF may be overwritten by the next tile's second G4
-      {                                                // chunked order: a warp stores 512 contiguous bytes per instruction
-        uint4* dst = reinterpret_cast<uint4*>(P.dthat) + ((bz * ntiles + ct) * C::NQ + cq) * 4 * ROWS + row;
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-          uint4 u;
-          __half2* h2 = reinterpret_cast<__half2*>(&u);
-#pragma unroll
-          for (int t = 0; t < 4; ++t) h2[t] = __floats2half2_rn(v[q * 8 + 2 * t], v[q * 8 + 2 * t + 1]);
-          dst[q * ROWS] = u;
-        }
+      // one pass, one exchange: with g = gelu(m), n = (g - mu) rstd the row sums the LayerNorm backward needs are
+      //   sum_j dnb_j n_j = rstd (sum dnb g - mu sum dnb)   and   sum_j dnb_j
+      uint32_t dgh[16];                              // gelu', packed to fp16 inside the pass (dm is rounded to fp16 for the MMAs anyway)
+      uint32_t gh[16];                               // g, packed to fp16 once the row sums have seen it in fp32 (it only re-enters
+                                                     // through the small LayerNorm projection term of dm): 16 registers instead of 32
+      float st[4];
+      {
+        float st01[2];
+        gelu_rowsums32_stash(v, s_b3 + h * D + col0, dgh, st01);
+        st[0] = st01[0]; st[1] = st01[1];
       }
-      A_STAMP(32, 20);
+      // the cotangent rows were requested one phase ago; touching them only now keeps their L2 latency off the gelu pass
+      {
+        float2 s2 = tc::splat2(0.f), s3 = tc::splat2(0.f);
+#pragma unroll
+        for (int j4 = 0; j4 < 32; j4 += 4) {
+          const __half2* h2 = reinterpret_cast<const __half2*>(&dnq[j4 >> 3]) + ((j4 & 4) >> 1);     // dnb[j4 .. j4 + 3], packed
+          const float2 d01 = __half22float2(h2[0]), d23 = __half22float2(h2[1]);
+          s2 = tc::fma2(d01, tc::ld2(v + j4), s2); s3 = tc::add2(s3, d01);
+          s2 = tc::fma2(d23, tc::ld2(v + j4 + 2), s2); s3 = tc::add2(s3, d23);
+          gh[j4 >> 1] = tc::pack_bf16(v[j4], v[j4 + 1]);
+          gh[(j4 >> 1) + 1] = tc::pack_bf16(v[j4 + 2], v[j4 + 3]);
+        }
+        st[2] = s2.x + s2.y; st[3] = s3.x + s3.y;
+      }
+      row_exchange<C::NQ, 4>(s_exch, xw, cq, row, lq, st);
+      float att = 0.f, Dh = 0.f;
+      if (valid) {
+        const float* rs = s_rs + e * 3 * ROWS * H + row * H + h;
+        att = __expf(rs[0] - rs[ROWS * H]);
+        Dh = rs[2 * ROWS * H];
+      }
+      const float atts = att;                        // dnb16 already carries the scale gs
+      const float mu = st[0] * (1.f / D);
+      const float rstd = rsqrtf(fmaxf(st[1] * (1.f / D) - mu * mu, 0.f) + 1e-6f);
+      const float dd0 = rstd * (st[2] - mu * st[3]), dd1 = st[3];
+      const float dsh = atts * (dd0 - Dh * gs);
+      const float mean1 = atts * dd1 * (1.f / D), mean2 = atts * dd0 * (1.f / D);
+      // dm = rstd (att dnb - mean1 - n mean2) g'   with n = (g - mu) rstd, constants folded
+      const float ka = atts * rstd, kc = rstd * (mu * rstd * mean2 - mean1), kb = rstd * rstd * mean2;
+      uint8_t* sDh = sDm + h * C::ATILE;
+      if (h == 0 && ct > 0) tc::mbar_wait(bar_gb, par ^ 1);      // every MMA of the previous tile is done with the dm tiles
+      uint32_t dmh[16];                              // dm as the fp16 operand words the MMAs read; the bias column sums add the same words
+#pragma unroll
+      for (int c8 = 0; c8 < 32; c8 += 8) {
+        const __half2* h2 = reinterpret_cast<const __half2*>(&dnq[c8 >> 3]);
+        const __half2* g2 = reinterpret_cast<const __half2*>(&gh[c8 >> 1]);
+        const __half2* d2 = reinterpret_cast<const __half2*>(&dgh[c8 >> 1]);
+#pragma unroll
+        for (int t = 0; t < 4; ++t) {
+          const float2 dv = __half22float2(h2[t]), gv = __half22float2(g2[t]);
+          const float2 dm = tc::mul2(tc::fma2(gv, tc::splat2(-kb), tc::fma2(tc::splat2(ka), dv, tc::splat2(kc))), __half22float2(d2[t]));
+          dmh[(c8 >> 1) + t] = tc::pack_bf16(dm.x, dm.y);
+        }
+        tc::st_row8_words(sDh, C::ABLK, row, col0 + c8, dmh + (c8 >> 1));
+      }
+      tc::fence_proxy_async();
+      tc::tc_fence_before();
+      if (warp == 0) {
+        named_sync(kABarHead + h, C::NT);
+        if (tc::elect_one()) issue_head(ct, h);
+        __syncwarp();
+      } else {
+        named_arrive(kABarHead + h, C::NT);            // warp 0 takes it from here
+      }
+      // fetch the cotangent rows of the next (tile, head) now, a whole phase ahead of their use
+      if (h + 1 < H) load_dnb(ct, h + 1);
+      else if (ct + 1 < ntiles) load_dnb(ct + 1, 0);
+      {
+        float cs = warp_colsum32_h2(dmh, lane);
+        atomicAdd(&s_db3[h * D + col0 + lane], cs);
+      }
+      if (cq == 0 && valid) P.ds[((bz * P.C) + c0 + row) * H + h] = dsh;
     }
-    tc::mbar_wait(bar_gb, (ntiles - 1) & 1);
+    // dthat = sum_h dm_h W3_h^T -> global (fp16, scaled)
+    tc::mbar_wait(bar_d, par);
     tc::tc_fence_after();
+    tc::tmem_ld32(tF + my_t, v);
+    tc::tmem_ld_wait();
+    tc::tc_fence_before();
+    if (ct + 1 < ntiles && warp != 0) named_arrive(kABarDth, C::NT);     // tF may be overwritten by the next tile's second G4
+    {                                                // chunked order: a warp stores 512 contiguous bytes per instruction
+      uint4* dst = reinterpret_cast<uint4*>(P.dthat) + ((bz * ntiles + ct) * C::NQ + cq) * 4 * ROWS + row;
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        uint4 u;
+        __half2* h2 = reinterpret_cast<__half2*>(&u);
+#pragma unroll
+        for (int t = 0; t < 4; ++t) h2[t] = __floats2half2_rn(v[q * 8 + 2 * t], v[q * 8 + 2 * t + 1]);
+        dst[q * ROWS] = u;
+      }
+    }
   }
+  tc::mbar_wait(bar_gb, (ntiles - 1) & 1);
+  tc::tc_fence_after();
   // flush dW3[b,z,h] (lane = input feature, column = output feature) and db3
   __syncthreads();
   tc::tc_fence_after();
-  if (!issuer) {
-    // accumulator row (input feature) of this thread (enf_pairs_tc_common.cuh: wgrad_row)
-    const int wrow = wgrad_row<D>(row, lq, lane);
+  // accumulator row (input feature) of this thread (enf_pairs_tc_common.cuh: wgrad_row)
+  const int wrow = wgrad_row<D>(row, lq, lane);
 #pragma unroll
-    for (int h = 0; h < H; ++h) {
-      float w[32];
-      tc::tmem_ld32(tW3 + h * D + my_t, w);
-      tc::tmem_ld_wait();
-      if (wrow >= 0) {
-        float* o = P.g_W3 + ((bz * H + h) * D + wrow) * D + col0;
+  for (int h = 0; h < H; ++h) {
+    float w[32];
+    tc::tmem_ld32(tW3 + h * D + my_t, w);
+    tc::tmem_ld_wait();
+    if (wrow >= 0) {
+      float* o = P.g_W3 + ((bz * H + h) * D + wrow) * D + col0;
 #pragma unroll
-        for (int j = 0; j < 32; j += 4)
-          *reinterpret_cast<float4*>(o + j) = make_float4(w[j] * inv_gs, w[j + 1] * inv_gs, w[j + 2] * inv_gs, w[j + 3] * inv_gs);
-      }
+      for (int j = 0; j < 32; j += 4)
+        *reinterpret_cast<float4*>(o + j) = make_float4(w[j] * inv_gs, w[j + 1] * inv_gs, w[j + 2] * inv_gs, w[j + 3] * inv_gs);
     }
   }
-  for (int e = tid; e < H * D; e += NTA) P.g_b3[bz * H * D + e] = s_db3[e] * inv_gs;
+  for (int e = tid; e < H * D; e += C::NT) P.g_b3[bz * H * D + e] = s_db3[e] * inv_gs;
   tc::tc_fence_before();
   __syncthreads();
   if (warp == 0) tc::tmem_dealloc<kTmemCols>(tm);
@@ -464,10 +419,9 @@ template <int D, int H>
 int launch_main(cudaStream_t st, const EnfPairTcBwdParams& p) {
   using C = BwdCfg<D, H>;
   size_t smem_a = ACfg<D, H>::SMEM_BYTES;
-  constexpr bool kSepIssueWarp = false;
-  if (cudaFuncSetAttribute(pairs_bwd_tc_a_kernel<D, H, kSepIssueWarp>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_a) != cudaSuccess) return -1;
+  if (cudaFuncSetAttribute(pairs_bwd_tc_a_kernel<D, H>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_a) != cudaSuccess) return -1;
   const unsigned grid = (unsigned)(p.B * p.Z);
-  pairs_bwd_tc_a_kernel<D, H, kSepIssueWarp><<<grid, C::NT + (kSepIssueWarp ? 32 : 0), smem_a, st>>>(p);
+  pairs_bwd_tc_a_kernel<D, H><<<grid, C::NT, smem_a, st>>>(p);
   if (enf_launch_pairs_bwd_tc_v(st, D, p) < 0) return -1;
   if (enf_launch_pairs_bwd_tc_q(st, D, H, p) < 0) return -1;
   return 3;

@@ -76,14 +76,6 @@ __device__ __forceinline__ void issue_du(uint32_t d_tmem, uint32_t a_addr, uint3
   for (int kk = 0; kk < HD / 16; ++kk) tc::mma_f16(d_tmem, tc::desc_kmajor(a_addr + kk * 32), tc::desc_kmajor(b_addr + kk * 32), idesc, kk > 0);
 }
 
-// diagnostics (build with `make TRACE=1`, run with ENF_DEBUG_TRACE=1): clock64() of selected events of CTA 7, its first
-// item, tiles 4..7, for thread `who`
-#ifdef ENF_TRACE
-#define Q_STAMP(who, slot) do { if (P.dbg && blockIdx.x == 7 && item == 7 && tid == (who) && ct >= 4 && ct < 8) P.dbg[1024 + ((who) == 32 ? 0 : 128) + (ct - 4) * 32 + (slot)] = clock64(); } while (0)
-#else
-#define Q_STAMP(who, slot) do { } while (0)
-#endif
-
 template <int D, int H>
 __global__ void __launch_bounds__(QCfg<D, H>::NTALL, D <= 64 ? 2 : 1) pairs_bwd_tc_q_kernel(EnfPairTcBwdParams P) {
   using C = QCfg<D, H>;
@@ -301,28 +293,21 @@ __global__ void __launch_bounds__(QCfg<D, H>::NTALL, D <= 64 ? 2 : 1) pairs_bwd_
       float pre8[8];                                       // cq == 0: xi of tile ct + 1 ; cq == 1, 2: du_v of tile ct - 1
       if (cq == 0) { if (ct + 1 < ntiles) load_xi(ct + 1, pre8); }
       else if (cq == kPart0 || cq == kPart1) { if (ct > 0) load_duv(ct - 1, pre8); }
-      Q_STAMP(32, 0); Q_STAMP(160, 0);
       if (it > 0) tc::mbar_wait(bar_u, (it - 1) & 1);     // every MMA of the previous tile is done with the operand tiles
-      Q_STAMP(32, 1); Q_STAMP(160, 1);
       // ---- S1: gamma_q hi / lo ---------------------------------------------------------------------------------
       tc::mbar_wait(bar_p, par);
       tc::tc_fence_after();
-      Q_STAMP(32, 2); Q_STAMP(160, 2);
       if (main_thr) rff_from_proj<D, true>(tP + lane_off + 16 * cq, sGhi, sGlo, C::ABLK, row, 16 * cq);
-      Q_STAMP(32, 3); Q_STAMP(160, 3);
       tc::tc_fence_before();
       tc::fence_proxy_async();
       __syncthreads();
-      Q_STAMP(32, 4); Q_STAMP(160, 4);
       if (warp == (MMA_TID >> 5)) {
         if (tc::elect_one()) {
           if (it == 0) tc::mbar_wait(bar_w, 0);
           tc::tc_fence_after();
           issue_gemm<D>(tT, aGhi, aW, C::ABLK, C::WBLK);
-          if (!P.debug_nosplit) {
-            issue_gemm<D>(tT, aGlo, aW, C::ABLK, C::WBLK, 1);
-            issue_gemm<D>(tT, aGhi, aWlo, C::ABLK, C::WBLK, 1);
-          }
+          issue_gemm<D>(tT, aGlo, aW, C::ABLK, C::WBLK, 1);
+          issue_gemm<D>(tT, aGhi, aWlo, C::ABLK, C::WBLK, 1);
           tc::mma_commit(bar_g1);
         }
         __syncwarp();
@@ -360,10 +345,8 @@ __global__ void __launch_bounds__(QCfg<D, H>::NTALL, D <= 64 ? 2 : 1) pairs_bwd_
       // ---- E: h1q, dzq ---------------------------------------------------------------------------------------------
       if (main_thr) {
       float v[32];
-      Q_STAMP(32, 5); Q_STAMP(160, 5);
       tc::mbar_wait(bar_g1, par);
       tc::tc_fence_after();
-      Q_STAMP(32, 6); Q_STAMP(160, 6);
       tc::tmem_ld32(tT + my_t, v);
       tc::tmem_ld_wait();
 #pragma unroll
@@ -389,7 +372,6 @@ __global__ void __launch_bounds__(QCfg<D, H>::NTALL, D <= 64 ? 2 : 1) pairs_bwd_
         tc::st_row8_bf16(sGlo, C::ABLK, row, col0 + c8, oh);
         tc::st_row8_bf16(sDz, C::ABLK, row, col0 + c8, oz);
       }
-      Q_STAMP(32, 7); Q_STAMP(160, 7);
       if (ct + 1 < ntiles) {
 #pragma unroll
         for (int h = 0; h < H; ++h) dsv_next[h] = (c0 + ROWS + row < P.C) ? __ldg(P.ds + (pr + ROWS) * H + h) : 0.f;
@@ -398,7 +380,6 @@ __global__ void __launch_bounds__(QCfg<D, H>::NTALL, D <= 64 ? 2 : 1) pairs_bwd_
       tc::tc_fence_before();
       tc::fence_proxy_async();
       __syncthreads();
-      Q_STAMP(32, 8); Q_STAMP(160, 8);
       if (warp == (MMA_TID >> 5)) {
         if (tc::elect_one()) {
           tc::tc_fence_after();
@@ -422,7 +403,6 @@ __global__ void __launch_bounds__(QCfg<D, H>::NTALL, D <= 64 ? 2 : 1) pairs_bwd_
       if (main_thr) {
       tc::mbar_wait(bar_d, par);
       tc::tc_fence_after();
-      Q_STAMP(32, 9); Q_STAMP(160, 9);
       {
         float dsn[16], dcs[16];
         tc::tmem_ld16(tT + lane_off + 16 * cq, dsn);
@@ -445,11 +425,9 @@ __global__ void __launch_bounds__(QCfg<D, H>::NTALL, D <= 64 ? 2 : 1) pairs_bwd_
         }
       }
       }   // main_thr
-      Q_STAMP(32, 10); Q_STAMP(160, 10);
       tc::tc_fence_before();
       tc::fence_proxy_async();
       __syncthreads();
-      Q_STAMP(32, 11); Q_STAMP(160, 11);
       if (warp == (MMA_TID >> 5)) {
         if (tc::elect_one()) {
           tc::tc_fence_after();

@@ -76,14 +76,6 @@ __device__ __forceinline__ void issue_du_v(uint32_t d_tmem, uint32_t a_addr, uin
   for (int kk = 0; kk < HD / 16; ++kk) tc::mma_f16(d_tmem, tc::desc_kmajor(a_addr + kk * 32), tc::desc_kmajor(b_addr + kk * 32), idesc, kk > 0);
 }
 
-// diagnostics (build with `make TRACE=1`, run with ENF_DEBUG_TRACE=1): clock64() of selected events of CTA 7, its first
-// item, tiles 4..7, for thread `who`
-#ifdef ENF_TRACE
-#define V_STAMP(slot) do { if (P.dbg && blockIdx.x == 7 && item == 7 && (tid == 32 || tid == 160) && ct >= 4 && ct < 8) P.dbg[2048 + (tid == 32 ? 0 : 128) + (ct - 4) * 32 + (slot)] = clock64(); } while (0)
-#else
-#define V_STAMP(slot) do { } while (0)
-#endif
-
 template <int D>
 __global__ void __launch_bounds__(VCfg<D>::NT, D == 32 ? 2 : 1) pairs_bwd_tc_v_kernel(EnfPairTcBwdParams P) {
   using C = VCfg<D>;
@@ -227,7 +219,6 @@ __global__ void __launch_bounds__(VCfg<D>::NT, D == 32 ? 2 : 1) pairs_bwd_tc_v_k
 #pragma unroll
         for (int q = 0; q < 4; ++q) dthq[q] = valid ? __ldg(src + q * ROWS) : make_uint4(0u, 0u, 0u, 0u);
       }
-      V_STAMP(0);
       if (it > 0) {                                        // every MMA of the previous tile is done with the operand tiles
         tc::mbar_wait(bar_u, (it - 1) & 1);
         tc::tc_fence_after();
@@ -238,10 +229,8 @@ __global__ void __launch_bounds__(VCfg<D>::NT, D == 32 ? 2 : 1) pairs_bwd_tc_v_k
       }
       if (cq == C::kDuCq && ct > 0) store_du(ct - 1, (it - 1) & 1);      // previous tile's du -> duv (the item's last tile: at its flush)
       // ---- S1: gamma_v hi / lo ---------------------------------------------------------------------------------
-      V_STAMP(1);
       tc::mbar_wait(bar_p, par);
       tc::tc_fence_after();
-      V_STAMP(2);
       // sin half first: the K-steps over the sin features (3 split terms) are issued as soon as that half is written
       // (named barrier 5: the issuing warp syncs, the others arrive) and run in the shadow of the cos half
       constexpr int KH = D / 32;                           // K-steps (16 features) per half of gamma
@@ -253,10 +242,8 @@ __global__ void __launch_bounds__(VCfg<D>::NT, D == 32 ? 2 : 1) pairs_bwd_tc_v_k
           if (it == 0) tc::mbar_wait(bar_w, 0);
           tc::tc_fence_after();
           issue_gemm_ksteps<D>(tT, aGhi, aW, C::ABLK, C::WBLK, 0, KH, 0);
-          if (!P.debug_nosplit) {
-            issue_gemm_ksteps<D>(tT, aX, aW, C::ABLK, C::WBLK, 0, KH, 1);
-            issue_gemm_ksteps<D>(tT, aGhi, aWlo, C::ABLK, C::WBLK, 0, KH, 1);
-          }
+          issue_gemm_ksteps<D>(tT, aX, aW, C::ABLK, C::WBLK, 0, KH, 1);
+          issue_gemm_ksteps<D>(tT, aGhi, aWlo, C::ABLK, C::WBLK, 0, KH, 1);
         }
         __syncwarp();
       } else {
@@ -269,18 +256,14 @@ __global__ void __launch_bounds__(VCfg<D>::NT, D == 32 ? 2 : 1) pairs_bwd_tc_v_k
       }
       const float trs = valid ? __ldg(P.trstd + (size_t)bz * ntiles * ROWS + c0 + row) : 0.f;
       rff_half_from_proj<D, true, false>(tP + lane_off + 16 * cq, sGhi, sX, C::ABLK, row, 16 * cq);
-      V_STAMP(3);
       tc::tc_fence_before();
       tc::fence_proxy_async();
       __syncthreads();
-      V_STAMP(4);
       if (tid == MMA_TID) {
         tc::tc_fence_after();
         issue_gemm_ksteps<D>(tT, aGhi, aW, C::ABLK, C::WBLK, KH, 2 * KH, 1);
-        if (!P.debug_nosplit) {
-          issue_gemm_ksteps<D>(tT, aX, aW, C::ABLK, C::WBLK, KH, 2 * KH, 1);
-          issue_gemm_ksteps<D>(tT, aGhi, aWlo, C::ABLK, C::WBLK, KH, 2 * KH, 1);
-        }
+        issue_gemm_ksteps<D>(tT, aX, aW, C::ABLK, C::WBLK, KH, 2 * KH, 1);
+        issue_gemm_ksteps<D>(tT, aGhi, aWlo, C::ABLK, C::WBLK, KH, 2 * KH, 1);
         tc::mma_commit(bar_g1);
       }
       // ---- in the shadow of the 3-term GEMM: E3 and the next tile's invariants -----------------------------------------
@@ -331,10 +314,8 @@ __global__ void __launch_bounds__(VCfg<D>::NT, D == 32 ? 2 : 1) pairs_bwd_tc_v_k
       if (cq == 0 && ct + 1 < ntiles) write_invariants(xi_next);
       // ---- E2: h1v, mask ---------------------------------------------------------------------------------------------
       float v[32];
-      V_STAMP(5);
       tc::mbar_wait(bar_g1, par);
       tc::tc_fence_after();
-      V_STAMP(6);
       tc::tmem_ld32(tT + my_t, v);
       tc::tmem_ld_wait();
       uint32_t neg = 0;                                    // bit j: pre-activation j is negative (sign bits, two integer ops per element)
@@ -352,11 +333,9 @@ __global__ void __launch_bounds__(VCfg<D>::NT, D == 32 ? 2 : 1) pairs_bwd_tc_v_k
         }
         tc::st_row8_bf16(sX, C::ABLK, row, col0 + c8, o);
       }
-      V_STAMP(7);
       tc::tc_fence_before();
       tc::fence_proxy_async();
       __syncthreads();
-      V_STAMP(8);
       if (tid == MMA_TID) {
         tc::tc_fence_after();
         issue_dgrad<D>(tT, aDt, aWp, C::ABLK, C::WBLK, 0);          // d h1v
@@ -371,25 +350,19 @@ __global__ void __launch_bounds__(VCfg<D>::NT, D == 32 ? 2 : 1) pairs_bwd_tc_v_k
           tc::mma_commit(bar_p);
         }
       }
-      V_STAMP(9); V_STAMP(10); V_STAMP(11);
       // ---- E4: dzv = d h1v [h1v > 0] ----------------------------------------------------------------------------------
       tc::mbar_wait(bar_g3, par);
       tc::tc_fence_after();
-      V_STAMP(12);
       tc::tmem_ld32(tT + my_t, v);
       tc::tmem_ld_wait();
 #pragma unroll
       for (int j = 0; j < 32; ++j) v[j] = ((neg >> j) & 1u) ? 0.f : v[j];
-      V_STAMP(13);
       tc::mbar_wait(bar_g3b, par);                         // the wgrad has finished reading dtpre: its tile takes dzv
-      V_STAMP(14);
 #pragma unroll
       for (int c8 = 0; c8 < 32; c8 += 8) tc::st_row8_bf16(sDt, C::ABLK, row, col0 + c8, v + c8);
-      V_STAMP(15);
       tc::tc_fence_before();
       tc::fence_proxy_async();
       __syncthreads();
-      V_STAMP(16);
       if (tid == MMA_TID) {
         tc::tc_fence_after();
         issue_dgrad<D>(tT, aDt, aW, C::ABLK, C::WBLK, 0);           // d gamma_v
@@ -402,7 +375,6 @@ __global__ void __launch_bounds__(VCfg<D>::NT, D == 32 ? 2 : 1) pairs_bwd_tc_v_k
       // ---- S3: d gamma_v -> dproj (my 16 frequencies: sin columns j, cos columns HD + j) ---------------------------
       tc::mbar_wait(bar_g4, par);
       tc::tc_fence_after();
-      V_STAMP(17);
       {
         float dsn[16], dcs[16];
         tc::tmem_ld16(tT + lane_off + 16 * cq, dsn);
@@ -425,11 +397,9 @@ __global__ void __launch_bounds__(VCfg<D>::NT, D == 32 ? 2 : 1) pairs_bwd_tc_v_k
           tc::st_row8_bf16(sX, C::ABLK, row, col, o);               // h1v's wgrad completed before E4 stored (bar_g3b)
         }
       }
-      V_STAMP(18);
       tc::tc_fence_before();
       tc::fence_proxy_async();
       __syncthreads();
-      V_STAMP(19);
       if (tid == MMA_TID) {
         tc::tc_fence_after();
         issue_du_v<HD>(tDu, aX, aOmT);

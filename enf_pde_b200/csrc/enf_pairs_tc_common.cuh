@@ -33,67 +33,9 @@ __device__ __forceinline__ float tanh_fast(float x) {
   asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
   return y;
 }
-// jax.nn.gelu(approximate=True) and its derivative, sharing one tanh
-__device__ __forceinline__ float gelu_fast(float x) {
-  const float c0 = 0.7978845608028654f, c1 = 0.7978845608028654f * 0.044715f;
-  float t = tanh_fast(x * fmaf(c1, x * x, c0));
-  return x * fmaf(0.5f, t, 0.5f);               // same expression as gelu_fast_both: the backward's recompute matches bit for bit
-}
-__device__ __forceinline__ void gelu_fast_both(float x, float& g, float& dg) {
-  const float c0 = 0.7978845608028654f, c1 = 0.7978845608028654f * 0.044715f;
-  float x2 = x * x;
-  float t = tanh_fast(x * fmaf(c1, x2, c0));
-  float s = fmaf(0.5f, t, 0.5f);                 // 0.5 (1 + t)
-  g = x * s;
-  // d/dx = s + x * 0.5 (1 - t^2) (c0 + 3 c1 x^2),  0.5 (1 - t^2) = s (2 - 2 s)  =>  s + g (2 - 2 s) (c0 + 3 c1 x^2)
-  dg = fmaf(g * fmaf(-2.f, s, 2.f), fmaf(3.f * c1, x2, c0), s);
-}
-
-// the same two functions on a pair of elements: FFMA2 / FMUL2 (tc::fma2 / mul2), each lane bit-identical to the scalar code above
-__device__ __forceinline__ float2 gelu_fast2(float2 x) {
-  const float c0 = 0.7978845608028654f, c1 = 0.7978845608028654f * 0.044715f;
-  const float2 x2 = tc::mul2(x, x);
-  const float2 a = tc::mul2(x, tc::fma2(tc::splat2(c1), x2, tc::splat2(c0)));
-  const float2 t = make_float2(tanh_fast(a.x), tanh_fast(a.y));
-  return tc::mul2(x, tc::fma2(tc::splat2(0.5f), t, tc::splat2(0.5f)));
-}
-__device__ __forceinline__ void gelu_fast_both2(float2 x, float2& g, float2& dg) {
-  const float c0 = 0.7978845608028654f, c1 = 0.7978845608028654f * 0.044715f;
-  const float2 x2 = tc::mul2(x, x);
-  const float2 a = tc::mul2(x, tc::fma2(tc::splat2(c1), x2, tc::splat2(c0)));
-  const float2 t = make_float2(tanh_fast(a.x), tanh_fast(a.y));
-  const float2 s = tc::fma2(tc::splat2(0.5f), t, tc::splat2(0.5f));
-  g = tc::mul2(x, s);
-  dg = tc::fma2(tc::mul2(g, tc::fma2(tc::splat2(-2.f), s, tc::splat2(2.f))), tc::fma2(tc::splat2(3.f * c1), x2, tc::splat2(c0)), s);
-}
-
-// Two independent pairs at once, written stage by stage: ptxas keeps the source order of these chains when registers are
-// tight (it otherwise runs one dependent FMUL2 -> FFMA2 -> FMUL2 -> MUFU -> FFMA2 -> FMUL2 chain after the other, 45
-// cycles of latency per pair with nothing of the same warp to fill it).
-__device__ __forceinline__ void gelu_fast2x2(float2 xa, float2 xb, float2& ga, float2& gb) {
-  const float c0 = 0.7978845608028654f, c1 = 0.7978845608028654f * 0.044715f;
-  float2 pa = tc::mul2(xa, xa), pb = tc::mul2(xb, xb);
-  pa = tc::fma2(tc::splat2(c1), pa, tc::splat2(c0)); pb = tc::fma2(tc::splat2(c1), pb, tc::splat2(c0));
-  pa = tc::mul2(xa, pa); pb = tc::mul2(xb, pb);
-  pa.x = tanh_fast(pa.x); pb.x = tanh_fast(pb.x); pa.y = tanh_fast(pa.y); pb.y = tanh_fast(pb.y);
-  pa = tc::fma2(tc::splat2(0.5f), pa, tc::splat2(0.5f)); pb = tc::fma2(tc::splat2(0.5f), pb, tc::splat2(0.5f));
-  ga = tc::mul2(xa, pa); gb = tc::mul2(xb, pb);
-}
-__device__ __forceinline__ void gelu_fast_both2x2(float2 xa, float2 xb, float2& ga, float2& gb, float2& dga, float2& dgb) {
-  const float c0 = 0.7978845608028654f, c1 = 0.7978845608028654f * 0.044715f;
-  const float2 x2a = tc::mul2(xa, xa), x2b = tc::mul2(xb, xb);
-  float2 pa = tc::fma2(tc::splat2(c1), x2a, tc::splat2(c0)), pb = tc::fma2(tc::splat2(c1), x2b, tc::splat2(c0));
-  pa = tc::mul2(xa, pa); pb = tc::mul2(xb, pb);
-  pa.x = tanh_fast(pa.x); pb.x = tanh_fast(pb.x); pa.y = tanh_fast(pa.y); pb.y = tanh_fast(pb.y);
-  const float2 sa = tc::fma2(tc::splat2(0.5f), pa, tc::splat2(0.5f)), sb = tc::fma2(tc::splat2(0.5f), pb, tc::splat2(0.5f));
-  ga = tc::mul2(xa, sa); gb = tc::mul2(xb, sb);
-  const float2 ra = tc::fma2(tc::splat2(3.f * c1), x2a, tc::splat2(c0)), rb = tc::fma2(tc::splat2(3.f * c1), x2b, tc::splat2(c0));
-  const float2 qa = tc::mul2(ga, tc::fma2(tc::splat2(-2.f), sa, tc::splat2(2.f))), qb = tc::mul2(gb, tc::fma2(tc::splat2(-2.f), sb, tc::splat2(2.f)));
-  dga = tc::fma2(qa, ra, sa); dgb = tc::fma2(qb, rb, sb);
-}
 
 // v[j] <- g_j = gelu(v[j] + bias[j]) over a thread's 32 columns (bias: 16-byte aligned, shared memory); st = {sum g, sum g^2}
-// (even / odd partial sums).  The LayerNorm statistics of the forward (E3, E4) in packed form, eight columns at a time and
+// (even / odd partial sums); gelu is jax.nn.gelu(approximate=True).  The LayerNorm statistics of the forward (E3, E4) in packed form, eight columns at a time and
 // stage by stage, so that four independent chains (and their eight MUFU.TANH) are in flight per warp.
 __device__ __forceinline__ void gelu_rowsums32(float (&v)[32], const float* bias, float (&st)[2]) {
   const float c0 = 0.7978845608028654f, c1 = 0.7978845608028654f * 0.044715f;
@@ -116,38 +58,6 @@ __device__ __forceinline__ void gelu_rowsums32(float (&v)[32], const float* bias
     for (int i = 0; i < 4; ++i) p[i] = tc::fma2(tc::splat2(0.5f), p[i], tc::splat2(0.5f));
 #pragma unroll
     for (int i = 0; i < 4; ++i) { x[i] = tc::mul2(x[i], p[i]); tc::st2(v + c8 + 2 * i, x[i]); }
-#pragma unroll
-    for (int i = 0; i < 4; ++i) { s0 = tc::add2(s0, x[i]); s1 = tc::fma2(x[i], x[i], s1); }
-  }
-  st[0] = s0.x + s0.y; st[1] = s1.x + s1.y;
-}
-
-// Same pass for the backward kernels: v[j] <- g_j, dg[j] <- gelu'(v[j] + bias[j]); st[0] = sum g, st[1] = sum g^2.
-__device__ __forceinline__ void gelu_both_rowsums32(float (&v)[32], const float* bias, float (&dg)[32], float (&st)[4]) {
-  const float c0 = 0.7978845608028654f, c1 = 0.7978845608028654f * 0.044715f;
-  float2 s0 = tc::splat2(0.f), s1 = tc::splat2(0.f);
-#pragma unroll
-  for (int c8 = 0; c8 < 32; c8 += 8) {
-    const float4 b0 = *reinterpret_cast<const float4*>(bias + c8), b1 = *reinterpret_cast<const float4*>(bias + c8 + 4);
-    float2 x[4], x2[4], p[4];
-    x[0] = tc::add2(tc::ld2(v + c8), make_float2(b0.x, b0.y)); x[1] = tc::add2(tc::ld2(v + c8 + 2), make_float2(b0.z, b0.w));
-    x[2] = tc::add2(tc::ld2(v + c8 + 4), make_float2(b1.x, b1.y)); x[3] = tc::add2(tc::ld2(v + c8 + 6), make_float2(b1.z, b1.w));
-#pragma unroll
-    for (int i = 0; i < 4; ++i) x2[i] = tc::mul2(x[i], x[i]);
-#pragma unroll
-    for (int i = 0; i < 4; ++i) p[i] = tc::fma2(tc::splat2(c1), x2[i], tc::splat2(c0));
-#pragma unroll
-    for (int i = 0; i < 4; ++i) p[i] = tc::mul2(x[i], p[i]);
-#pragma unroll
-    for (int i = 0; i < 4; ++i) { p[i].x = tanh_fast(p[i].x); p[i].y = tanh_fast(p[i].y); }
-#pragma unroll
-    for (int i = 0; i < 4; ++i) x2[i] = tc::fma2(tc::splat2(3.f * c1), x2[i], tc::splat2(c0));      // in the shadow of the tanh
-#pragma unroll
-    for (int i = 0; i < 4; ++i) p[i] = tc::fma2(tc::splat2(0.5f), p[i], tc::splat2(0.5f));          // s
-#pragma unroll
-    for (int i = 0; i < 4; ++i) { x[i] = tc::mul2(x[i], p[i]); tc::st2(v + c8 + 2 * i, x[i]); }       // g
-#pragma unroll
-    for (int i = 0; i < 4; ++i) tc::st2(dg + c8 + 2 * i, tc::fma2(tc::mul2(x[i], tc::fma2(tc::splat2(-2.f), p[i], tc::splat2(2.f))), x2[i], p[i]));
 #pragma unroll
     for (int i = 0; i < 4; ++i) { s0 = tc::add2(s0, x[i]); s1 = tc::fma2(x[i], x[i], s1); }
   }
@@ -188,42 +98,6 @@ __device__ __forceinline__ void gelu_rowsums32_stash(float (&v)[32], const float
     for (int i = 0; i < 4; ++i) { s0 = tc::add2(s0, x[i]); s1 = tc::fma2(x[i], x[i], s1); }
   }
   st[0] = s0.x + s0.y; st[1] = s1.x + s1.y;
-}
-
-// Eight columns of the LayerNorm / gelu backward's first pass with everything it feeds folded in (register-minimal form of
-// the pass above): x = v + bias; g = gelu(x) -> gh (packed fp16, after the row sums have seen it in fp32); dg = gelu'(x);
-// s0 += g, s1 += g^2, s2 += dth g, s3 += dth, with dth the (packed fp16) cotangent of the LayerNorm output.
-__device__ __forceinline__ void gelu_both_stats8(const float* v, const float* bias, const uint4& dth, float* dg, uint32_t* gh, float2& s0,
-                                                 float2& s1, float2& s2, float2& s3) {
-  const float c0 = 0.7978845608028654f, c1 = 0.7978845608028654f * 0.044715f;
-  const float4 b0 = *reinterpret_cast<const float4*>(bias), b1 = *reinterpret_cast<const float4*>(bias + 4);
-  float2 x[4], x2[4], p[4];
-  x[0] = tc::add2(tc::ld2(v), make_float2(b0.x, b0.y)); x[1] = tc::add2(tc::ld2(v + 2), make_float2(b0.z, b0.w));
-  x[2] = tc::add2(tc::ld2(v + 4), make_float2(b1.x, b1.y)); x[3] = tc::add2(tc::ld2(v + 6), make_float2(b1.z, b1.w));
-#pragma unroll
-  for (int i = 0; i < 4; ++i) x2[i] = tc::mul2(x[i], x[i]);
-#pragma unroll
-  for (int i = 0; i < 4; ++i) p[i] = tc::fma2(tc::splat2(c1), x2[i], tc::splat2(c0));
-#pragma unroll
-  for (int i = 0; i < 4; ++i) p[i] = tc::mul2(x[i], p[i]);
-#pragma unroll
-  for (int i = 0; i < 4; ++i) { p[i].x = tanh_fast(p[i].x); p[i].y = tanh_fast(p[i].y); }
-#pragma unroll
-  for (int i = 0; i < 4; ++i) x2[i] = tc::fma2(tc::splat2(3.f * c1), x2[i], tc::splat2(c0));       // in the shadow of the tanh
-#pragma unroll
-  for (int i = 0; i < 4; ++i) p[i] = tc::fma2(tc::splat2(0.5f), p[i], tc::splat2(0.5f));          // s
-#pragma unroll
-  for (int i = 0; i < 4; ++i) x[i] = tc::mul2(x[i], p[i]);                                         // g
-#pragma unroll
-  for (int i = 0; i < 4; ++i) tc::st2(dg + 2 * i, tc::fma2(tc::mul2(x[i], tc::fma2(tc::splat2(-2.f), p[i], tc::splat2(2.f))), x2[i], p[i]));
-  const __half2* h2 = reinterpret_cast<const __half2*>(&dth);
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const float2 d = __half22float2(h2[i]);
-    s0 = tc::add2(s0, x[i]); s1 = tc::fma2(x[i], x[i], s1);
-    s2 = tc::fma2(d, x[i], s2); s3 = tc::add2(s3, d);
-    gh[i] = tc::pack_bf16(x[i].x, x[i].y);
-  }
 }
 
 // cos of two RFF phases on the FMA pipe (packed), so that the XU pipe (4 lanes per scheduler: a warp-wide MUFU takes 8
