@@ -85,10 +85,11 @@ FLAG_OUT_BF16 = 8
 FLAG_FROZEN_RELU = 16
 FLAG_SELF_BLOCK = 32
 FLAG_NO_STEM = 64
+FLAG_GRAD_X = 128
 ABI_VERSION = 2
 
 EXPORTS = ("enf_abi_version", "enf_invariant_dim", "enf_pose_dim", "enf_xattn_workspace_bytes", "enf_xattn_chunk_for_cap",
-           "enf_xattn_dispatch", "enf_workspace_release", "enf_xattn_fwd", "enf_xattn_bwd", "enf_last_launch_count",
+           "enf_xattn_dispatch", "enf_workspace_release", "enf_xattn_fwd", "enf_xattn_bwd", "enf_xattn_bwd_x", "enf_last_launch_count",
            "enf_last_error", "enf_debug_ws_offset", "enf_profile_enable", "enf_profile_collect", "enf_debug_tc_gemm",
            "enf_debug_gemm")
 
@@ -140,6 +141,9 @@ def load():
     lib.enf_xattn_bwd.restype = ctypes.c_int
     lib.enf_xattn_bwd.argtypes = [ctypes.POINTER(EnfDesc), ctypes.POINTER(EnfWeights), vp, i64, vp, vp, vp, vp,
                                   ctypes.POINTER(EnfWeights), vp, vp, vp, vp, ctypes.c_size_t, vp]
+    lib.enf_xattn_bwd_x.restype = ctypes.c_int
+    lib.enf_xattn_bwd_x.argtypes = [ctypes.POINTER(EnfDesc), ctypes.POINTER(EnfWeights), vp, i64, vp, vp, vp, vp,
+                                    ctypes.POINTER(EnfWeights), vp, vp, vp, vp, vp, ctypes.c_size_t, vp]
     lib.enf_last_launch_count.restype = ctypes.c_int
     lib.enf_last_error.restype = ctypes.c_char_p
     lib.enf_debug_ws_offset.restype = ctypes.c_int64

@@ -89,8 +89,11 @@ int validate(const EnfDesc* D, EnfRecordLayout* rl) {
   if ((int64_t)D->B * D->Z * D->H > 65535) return fail(ENF_ERR_UNSUPPORTED, "B*Z*H must be <= 65535 per call (shard the fields)");
   if (D->B > 65535) return fail(ENF_ERR_UNSUPPORTED, "B must be <= 65535");
   if (D->precision != ENF_PREC_FP32 && D->precision != ENF_PREC_BF16) return fail(ENF_ERR_BAD_DESC, "unknown precision");
-  if (D->flags & ~(ENF_FLAG_FORWARD_ONLY | ENF_FLAG_RECOMPUTE | ENF_FLAG_OUT_BF16 | ENF_FLAG_FROZEN_RELU | ENF_FLAG_SELF_BLOCK | ENF_FLAG_NO_STEM))
+  if (D->flags & ~(ENF_FLAG_FORWARD_ONLY | ENF_FLAG_RECOMPUTE | ENF_FLAG_OUT_BF16 | ENF_FLAG_FROZEN_RELU | ENF_FLAG_SELF_BLOCK | ENF_FLAG_NO_STEM |
+                   ENF_FLAG_GRAD_X))
     return fail(ENF_ERR_BAD_DESC, "unknown bits in flags");
+  if ((D->flags & ENF_FLAG_GRAD_X) && (D->flags & (ENF_FLAG_FORWARD_ONLY | ENF_FLAG_SELF_BLOCK)))
+    return fail(ENF_ERR_BAD_DESC, "ENF_FLAG_GRAD_X needs a backward (not ENF_FLAG_FORWARD_ONLY) of a decode call (not ENF_FLAG_SELF_BLOCK)");
   if ((D->flags & ENF_FLAG_NO_STEM) && D->L != D->d) return fail(ENF_ERR_BAD_DESC, "ENF_FLAG_NO_STEM: a is the hidden state, L must equal d");
   if (D->flags & ENF_FLAG_SELF_BLOCK) {
     if (D->C != D->Z || D->O != D->d) return fail(ENF_ERR_BAD_DESC, "ENF_FLAG_SELF_BLOCK: the queries are the latents (C == Z) and out is the hidden state (O == d)");
@@ -185,6 +188,7 @@ Layout make_layout(const EnfDesc& D, const EnfRecordLayout& rl) {
     return v;
   }();
   for (int i = 0; i < ENF_NUM_WEIGHT_LEAVES; ++i) Y.add(names[i].c_str(), n[i]);
+  if (D.flags & ENF_FLAG_GRAD_X) Y.add("g_xi", BC * ENF_F_XI);     // cotangent of the query records (reduced over latents)
   Y.acc_end = Y.total;
   return Y;
 }
@@ -323,6 +327,7 @@ void shift_fields(EnfPairTcBwdParams& tp, const EnfDesc& D, int b0, int nb) {
   tp.dnbar += bc * Hd; tp.Dg += bc * D.H; tp.dnb16 += (int64_t)b0 * ntiles * 128 * Hd / 8;
   tp.g_W3 += bz * D.H * (int64_t)D.d * D.d; tp.g_b3 += bz * Hd;
   tp.g_U += bz * Hd; tp.g_kappa += bz * D.H; tp.g_lam += bz * ENF_LAM_SIZE; tp.g_sigma += bz;
+  if (tp.g_xi) tp.g_xi += bc * ENF_F_XI;
 }
 
 // argument checks shared by enf_xattn_fwd and enf_xattn_bwd
@@ -607,9 +612,13 @@ int enf_xattn_fwd(const EnfDesc* desc, const EnfWeights* w, const float* x, int6
   return ENF_OK;
 }
 
-int enf_xattn_bwd(const EnfDesc* desc, const EnfWeights* w, const float* x, int64_t x_batch_stride, const float* p,
-                  const float* a, const float* sigma, const float* d_out, const EnfWeightGrads* dW, float* dp, float* da,
-                  float* dsigma, void* workspace, size_t workspace_bytes, enf_stream_t stream) {
+}  // extern "C"
+namespace {
+
+// enf_xattn_bwd (want_dx = false: dx is not computed, whatever the flags) and enf_xattn_bwd_x
+int xattn_bwd(const EnfDesc* desc, const EnfWeights* w, const float* x, int64_t x_batch_stride, const float* p,
+              const float* a, const float* sigma, const float* d_out, const EnfWeightGrads* dW, float* dp, float* da,
+              float* dsigma, float* dx, bool want_dx, void* workspace, size_t workspace_bytes, enf_stream_t stream) {
   g_launches = 0;
   EnfRecordLayout rl;
   int rc = validate(desc, &rl);
@@ -617,6 +626,10 @@ int enf_xattn_bwd(const EnfDesc* desc, const EnfWeights* w, const float* x, int6
   const EnfDesc& D = *desc;
   if (D.flags & ENF_FLAG_FORWARD_ONLY) return fail(ENF_ERR_STATE, "a forward-only description (ENF_FLAG_FORWARD_ONLY) has no backward");
   if (!d_out || !dp || !da) return fail(ENF_ERR_NULL_POINTER, "NULL argument");
+  if (want_dx && dx && !(D.flags & ENF_FLAG_GRAD_X))
+    return fail(ENF_ERR_STATE, "dx needs a forward run with ENF_FLAG_GRAD_X (its workspace holds the query-record cotangents)");
+  if (want_dx && !dx && (D.flags & ENF_FLAG_GRAD_X)) return fail(ENF_ERR_NULL_POINTER, "dx is NULL on an ENF_FLAG_GRAD_X description");
+  if (!want_dx) dx = nullptr;
   if ((rc = check_call(D, w, x, x_batch_stride, p, a, sigma, workspace)) != ENF_OK) return rc;
   {
     std::lock_guard<std::mutex> lk(g_mu);
@@ -744,6 +757,7 @@ int enf_xattn_bwd(const EnfDesc* desc, const EnfWeights* w, const float* x, int6
       tp.g_Wp = c.f("gf_Wp"); tp.g_bp = c.f("gf_bp");
     }
     tp.g_U = c.f("g_U"); tp.g_kappa = c.f("g_kappa"); tp.g_lam = c.f("g_lam"); tp.g_sigma = c.f("g_sigma");
+    tp.g_xi = dx ? c.f("g_xi") : nullptr;       // kernel C's GX variant
     prof_mark(1, 0, st);
     // once per backward: the power-of-two gradient scale, the fp16 cotangent of nbar in kernel A's load order, Dg
     nl = enf_launch_pairs_bwd_tc_prep(st, d, H, tp);
@@ -780,7 +794,7 @@ int enf_xattn_bwd(const EnfDesc* desc, const EnfWeights* w, const float* x, int6
     pp.g_Wp = c.f("gf_Wp"); pp.g_bp = c.f("gf_bp");
     pp.g_W3 = c.f("g_W3"); pp.g_b3 = c.f("g_b3"); pp.g_U = c.f("g_U"); pp.g_kappa = c.f("g_kappa");
     pp.g_lam = c.f("g_lam"); pp.g_sigma = c.f("g_sigma");
-    pp.g_xi = self ? c.f("g_xi") : nullptr;
+    pp.g_xi = (self || dx) ? c.f("g_xi") : nullptr;
     prof_mark(1, 0, st);
     nl = enf_launch_pairs_bwd_simt(st, d, pp);
     prof_mark(1, 1, st);
@@ -841,6 +855,7 @@ int enf_xattn_bwd(const EnfDesc* desc, const EnfWeights* w, const float* x, int6
     c.launches += enf_launch_pose_features_bwd(st, D.invariant_kind, D.Dx, rl.P, BZ, p, c.f("g_xi"), dp);
   } else {
     c.launches += enf_launch_latent_record_bwd(st, D, p, c.f("g_lam"), dp);
+    if (dx) c.launches += enf_launch_coord_features_bwd(st, D, x, Bx, c.f("g_xi"), dx);
   }
   if (dsigma) {
     if (cudaMemcpyAsync(dsigma, c.f("g_sigma"), BZ * sizeof(float), cudaMemcpyDeviceToDevice, st) != cudaSuccess)
@@ -927,6 +942,23 @@ int enf_xattn_bwd(const EnfDesc* desc, const EnfWeights* w, const float* x, int6
   if (e != cudaSuccess) return fail(ENF_ERR_CUDA, std::string("CUDA error while enqueueing bwd: ") + cudaGetErrorString(e));
   g_launches = c.launches;
   return ENF_OK;
+}
+
+}  // namespace
+extern "C" {
+
+int enf_xattn_bwd(const EnfDesc* desc, const EnfWeights* w, const float* x, int64_t x_batch_stride, const float* p,
+                  const float* a, const float* sigma, const float* d_out, const EnfWeightGrads* dW, float* dp, float* da,
+                  float* dsigma, void* workspace, size_t workspace_bytes, enf_stream_t stream) {
+  return xattn_bwd(desc, w, x, x_batch_stride, p, a, sigma, d_out, dW, dp, da, dsigma, nullptr, false, workspace, workspace_bytes,
+                   stream);
+}
+
+int enf_xattn_bwd_x(const EnfDesc* desc, const EnfWeights* w, const float* x, int64_t x_batch_stride, const float* p,
+                    const float* a, const float* sigma, const float* d_out, const EnfWeightGrads* dW, float* dp, float* da,
+                    float* dsigma, float* dx, void* workspace, size_t workspace_bytes, enf_stream_t stream) {
+  return xattn_bwd(desc, w, x, x_batch_stride, p, a, sigma, d_out, dW, dp, da, dsigma, dx, true, workspace, workspace_bytes,
+                   stream);
 }
 
 }  // extern "C"

@@ -129,6 +129,8 @@ int enf_launch_latent_record_bwd(cudaStream_t st, const EnfDesc& d, const float*
 // poses used as queries (latent ODE model: invariant(p, p)); self-attention variants of the invariants (ENF_INV_PONITA = Ponita2D, I = 3)
 int enf_launch_pose_features(cudaStream_t st, int kind, int Dx, int P, int64_t total, const float* p, float* xi);
 int enf_launch_pose_features_bwd(cudaStream_t st, int kind, int Dx, int P, int64_t total, const float* p, const float* dxi, float* dp);   // dp +=
+// decode queries: d(record) [B,C,8] -> dx [Bx,C,Dx] (overwritten; Bx = 1: a shared grid, summed over the B fields)
+int enf_launch_coord_features_bwd(cudaStream_t st, const EnfDesc& d, const float* x, int Bx, const float* dxi, float* dx);
 int enf_launch_pose_record(cudaStream_t st, int kind, int Dx, int P, int I, int64_t total, const float* p, float* lam);
 int enf_launch_pose_record_bwd(cudaStream_t st, int kind, int Dx, int P, int I, int win_kind, int64_t total, const float* p, const float* dlam, float* dp);   // dp =
 int enf_launch_weff(cudaStream_t st, const EnfDesc& d, const float* W2g, const float* b2g, const float* v0,
@@ -170,7 +172,7 @@ struct EnfPairParams {
   const float* slog;                         // [B,Z,C,H] logits saved by the tensor-core forward (or null: recompute)
   float* g_q_w1; float* g_q_b1; float* g_v_w1; float* g_v_b1; float* g_Wp; float* g_bp;   // accumulated (atomics)
   float* g_W3; float* g_b3; float* g_U; float* g_kappa; float* g_lam; float* g_sigma;      // per-latent, accumulated
-  float* g_xi;                               // [B,C,8] cotangent of the query records (self-attention blocks only), else null
+  float* g_xi;                               // [B,C,8] cotangent of the query records (self-attention blocks, ENF_FLAG_GRAD_X), else null
 };
 int enf_launch_pairs_fwd_simt(cudaStream_t st, int d, const EnfPairParams& p);
 int enf_launch_pairs_bwd_simt(cudaStream_t st, int d, const EnfPairParams& p);
@@ -223,6 +225,7 @@ struct EnfPairTcBwdParams {
   float* g_W3; float* g_b3;                  // per-latent outputs of A
   float* g_q_w1; float* g_q_b1; float* g_v_w1; float* g_v_b1; float* g_Wp; float* g_bp;   // shared-weight grads (atomics)
   float* g_U; float* g_kappa; float* g_lam; float* g_sigma;                                // per-latent outputs of B
+  float* g_xi;                               // [B,C,8] cotangent of the query records, accumulated by C (ENF_FLAG_GRAD_X), else null
 };
 bool enf_pairs_bwd_tc_supported(int d, int H);
 // prep (once per backward, whole batch): gradient scale, fp16 cotangent of nbar, Dg;  main: kernels A, B, C on p.B fields

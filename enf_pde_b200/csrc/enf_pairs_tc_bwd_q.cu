@@ -10,7 +10,8 @@
 //     S3  dproj_j = cos_j dsin_j - sin_j dcos_j  (thread-local: a thread owns sin AND cos of its 16 frequencies) -> tile
 //     M3  du = dproj Omega^T                  (N = 16: [Omega_hi | Omega_lo])
 //     S4  (one thread per row, overlapped with the next tile's M1) du += du_v (kernel B) ; window backward ;
-//         dq ; dLam += dq^T xi through a transposing butterfly ; dsigma
+//         dq ; dLam += dq^T xi through a transposing butterfly ; dsigma ; with GX also the cotangent of the row's query
+//         record, d xi += dq Lam (reduced over latents in global memory: one vector reduction per row thread and tile)
 // Every reduction over query rows that is a matrix product runs on the tensor core: column sums (bias gradient) and
 // ds-weighted column sums (dU) are `tile^T x S` MMAs against a [128 rows x 16] side operand S = [1 | ds_hi | ds_lo].
 // Shared-weight accumulators (dW1_q, db1q) live in TMEM for the CTA's whole life and are flushed once.
@@ -76,7 +77,13 @@ __device__ __forceinline__ void issue_du(uint32_t d_tmem, uint32_t a_addr, uint3
   for (int kk = 0; kk < HD / 16; ++kk) tc::mma_f16(d_tmem, tc::desc_kmajor(a_addr + kk * 32), tc::desc_kmajor(b_addr + kk * 32), idesc, kk > 0);
 }
 
-template <int D, int H>
+// *addr += (a, b, c, d) as one 16-byte reduction (addr 16-byte aligned)
+__device__ __forceinline__ void red_add_f32x4(float* addr, float a, float b, float c, float d) {
+  asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(addr), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
+}
+
+// GX: also reduce the cotangent of the query records into P.g_xi (ENF_FLAG_GRAD_X); false compiles to the plain backward
+template <int D, int H, bool GX>
 __global__ void __launch_bounds__(QCfg<D, H>::NTALL, D <= 64 ? 2 : 1) pairs_bwd_tc_q_kernel(EnfPairTcBwdParams P) {
   using C = QCfg<D, H>;
   constexpr int HD = C::HD;
@@ -245,6 +252,30 @@ __global__ void __launch_bounds__(QCfg<D, H>::NTALL, D <= 64 ? 2 : 1) pairs_bwd_
         if (r < P.I) {
           if (P.row_kind == ENF_ROW_SQDIST_SQRT) dq[r] = rec.u[r] > 0.f ? du[r] / (2.f * rec.u[r]) : 0.f;
           else dq[r] = du[r];
+        }
+      }
+      if constexpr (GX) {
+        // d xi[f] for my half of the record (part 0: f = 0..3, part 1: f = 4..7): DOT rows are bilinear in (Lam, xi),
+        // squared-distance rows (and the non-periodic window row) are sum_{f < nsq} (Lam_f - xi_f)^2, nsq <= 3
+        if (ct * ROWS + row < P.C) {
+          const float* Lp = s_lam + 4 * part;
+          float g[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+          for (int r = 0; r < ENF_R_LAM; ++r) {
+            if (r < P.I || (r == P.I && P.win_row >= 0)) {
+              const float* L = Lp + r * ENF_F_XI;
+              const bool sq = r < P.I ? (P.row_kind != ENF_ROW_DOT) : (P.win_kind == ENF_WIN_NP);
+              if (!sq) {
+#pragma unroll
+                for (int k = 0; k < 4; ++k) g[k] = fmaf(dq[r], L[k], g[k]);
+              } else if (part == 0) {
+#pragma unroll
+                for (int k = 0; k < 3; ++k) if (k < P.nsq) g[k] = fmaf(-2.f * dq[r], L[k] - xi_r[k], g[k]);
+              }
+            }
+          }
+          red_add_f32x4(P.g_xi + ((int64_t)b * P.C + ct * ROWS + row) * ENF_F_XI + 4 * part,
+                        g[0] * inv_gs, g[1] * inv_gs, g[2] * inv_gs, g[3] * inv_gs);
         }
       }
       float vv[32];
@@ -498,10 +529,10 @@ __global__ void __launch_bounds__(QCfg<D, H>::NTALL, D <= 64 ? 2 : 1) pairs_bwd_
   if (warp == 0) tc::tmem_dealloc<C::TMEM_COLS>(tm);
 }
 
-template <int D, int H>
+template <int D, int H, bool GX>
 int launch_q(cudaStream_t st, const EnfPairTcBwdParams& p) {
   using C = QCfg<D, H>;
-  if (cudaFuncSetAttribute(pairs_bwd_tc_q_kernel<D, H>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES) != cudaSuccess) return -1;
+  if (cudaFuncSetAttribute(pairs_bwd_tc_q_kernel<D, H, GX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES) != cudaSuccess) return -1;
   int nitems = p.B * p.Z;
   // persistent CTAs: as many as are resident at once.  TMEM (not visible to the occupancy API, which also under-reports
   // kernels with > 48 KB of dynamic shared memory: it answered 1 for d = 32 and halved the grid) allows 512 / TMEM_COLS
@@ -510,9 +541,11 @@ int launch_q(cudaStream_t st, const EnfPairTcBwdParams& p) {
   { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev); }
   const int ctas = occ * nsm;
   int grid = nitems < ctas ? nitems : ctas;
-  pairs_bwd_tc_q_kernel<D, H><<<grid, C::NTALL, C::SMEM_BYTES, st>>>(p);
+  pairs_bwd_tc_q_kernel<D, H, GX><<<grid, C::NTALL, C::SMEM_BYTES, st>>>(p);
   return 1;
 }
+template <int D, int H>
+int launch_q(cudaStream_t st, const EnfPairTcBwdParams& p) { return p.g_xi ? launch_q<D, H, true>(st, p) : launch_q<D, H, false>(st, p); }
 
 }  // namespace
 

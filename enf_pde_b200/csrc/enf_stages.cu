@@ -223,14 +223,9 @@ __global__ void latent_record_bwd_kernel(int kind, int Dx, int P, int I, int win
   for (int i = 0; i < P; ++i) dp[t * P + i] = g[i];
 }
 
-// d(xi record) -> d(raw pose) ACCUMULATED into dp, for poses used as queries (self-attention variant; rows of width P)
-__global__ void query_features_bwd_kernel(int kind, int Dx, int P, int64_t total, const float* __restrict__ p,
-                                          const float* __restrict__ dxi, float* __restrict__ dp) {
-  int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (t >= total) return;
-  const float* xr = p + t * P;
-  const float* d = dxi + t * ENF_F_XI;
-  float g[4] = {0.f, 0.f, 0.f, 0.f};
+// Adjoint of query_features_kernel for one row: g[0..3] = d(row xr) of the record cotangent d[8].  `sa`: the self-attention
+// variant (Ponita2D also reads the orientation xr[2]; coordinate rows of the ponita decode are only Dx = 2 wide).
+__device__ __forceinline__ void query_features_adjoint(int kind, int Dx, const float* xr, const float* d, float* g, bool sa) {
   switch (kind) {
     case ENF_INV_REL_POS: case ENF_INV_NORM_REL_POS: case ENF_INV_ABS_POS:
       for (int i = 0; i < Dx; ++i) g[i] = d[i];
@@ -242,8 +237,10 @@ __global__ void query_features_bwd_kernel(int kind, int Dx, int P, int64_t total
       }
       break;
     case ENF_INV_PONITA: {
-      float s, c; sincosf(xr[2], &s, &c);
-      g[0] = d[0]; g[1] = d[1]; g[2] = -s * d[3] + c * d[4];
+      float s = 0.f, c = 0.f;
+      if (sa) sincosf(xr[2], &s, &c);
+      g[0] = d[0]; g[1] = d[1];
+      if (sa) g[2] = -s * d[3] + c * d[4];
     } break;
     case ENF_INV_POLAR_PERIODIC: {
       float dphi[3], dth[3]; sph_unit_grad(xr[0], xr[1], dphi, dth);
@@ -263,7 +260,36 @@ __global__ void query_features_bwd_kernel(int kind, int Dx, int P, int64_t total
       g[2] = d[3];
     } break;
   }
+}
+
+// d(xi record) -> d(raw pose) ACCUMULATED into dp, for poses used as queries (self-attention variant; rows of width P)
+__global__ void query_features_bwd_kernel(int kind, int Dx, int P, int64_t total, const float* __restrict__ p,
+                                          const float* __restrict__ dxi, float* __restrict__ dp) {
+  int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= total) return;
+  float g[4] = {0.f, 0.f, 0.f, 0.f};
+  query_features_adjoint(kind, Dx, p + t * P, dxi + t * ENF_F_XI, g, true);
   for (int i = 0; i < P; ++i) dp[t * P + i] += g[i];
+}
+
+// d(xi record) [B,C,8] -> dx, OVERWRITTEN, for the coordinate queries of the decode (sa = 0).  One thread per row of x
+// (total = Bx*C rows of width Dx); nsum > 1 (shared grid, Bx = 1): the record cotangents of the nsum fields are summed first
+// (the record map is the same for every field, so the sum commutes with its adjoint).
+__global__ void coord_features_bwd_kernel(int kind, int Dx, int64_t total, int nsum, int64_t field_stride, const float* __restrict__ x,
+                                          const float* __restrict__ dxi, float* __restrict__ dx) {
+  int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= total) return;
+  float d[ENF_F_XI];
+#pragma unroll
+  for (int f = 0; f < ENF_F_XI; ++f) d[f] = 0.f;
+  for (int b = 0; b < nsum; ++b) {
+    const float4* src = reinterpret_cast<const float4*>(dxi + b * field_stride + t * ENF_F_XI);
+    const float4 u = src[0], v = src[1];
+    d[0] += u.x; d[1] += u.y; d[2] += u.z; d[3] += u.w; d[4] += v.x; d[5] += v.y; d[6] += v.z; d[7] += v.w;
+  }
+  float g[4] = {0.f, 0.f, 0.f, 0.f};
+  query_features_adjoint(kind, Dx, x + t * Dx, d, g, false);
+  for (int i = 0; i < Dx; ++i) dx[t * Dx + i] = g[i];
 }
 
 // ---- elementwise glue of the self-attention blocks (residual adds, the gelu between blocks; nef.py:62-64, 225-226) ------
@@ -748,6 +774,12 @@ int enf_launch_pose_features(cudaStream_t st, int kind, int Dx, int P, int64_t t
 }
 int enf_launch_pose_features_bwd(cudaStream_t st, int kind, int Dx, int P, int64_t total, const float* p, const float* dxi, float* dp) {
   query_features_bwd_kernel<<<blocks_for(total, 128), 128, 0, st>>>(kind, Dx, P, total, p, dxi, dp);
+  return 1;
+}
+int enf_launch_coord_features_bwd(cudaStream_t st, const EnfDesc& d, const float* x, int Bx, const float* dxi, float* dx) {
+  const int64_t total = (int64_t)Bx * d.C;
+  coord_features_bwd_kernel<<<blocks_for(total, 128), 128, 0, st>>>(d.invariant_kind, d.Dx, total, Bx == 1 ? d.B : 1,
+                                                                     (int64_t)d.C * ENF_F_XI, x, dxi, dx);
   return 1;
 }
 int enf_launch_pose_record(cudaStream_t st, int kind, int Dx, int P, int I, int64_t total, const float* p, float* lam) {

@@ -7,7 +7,9 @@
 
 `leaves` = the 46 arrays of `nef.init(...)['params']` in EnfWeights order (`enf_pde_b200._lib.LEAF_PATHS` maps each to its
 Flax path).  The op is once-differentiable (`jax.custom_vjp`): gradients w.r.t. leaves, p, a, sigma -- what `jax.grad` at
-pde_trainer.py:188,255 takes; coordinates get no gradient (the reference never differentiates them).
+pde_trainer.py:188,255 takes.  Known gap: the cotangent of the coordinates x is returned as zeros here.  The C ABI has it
+(ENF_FLAG_GRAD_X + enf_xattn_bwd_x, which the PyTorch binding uses), but the FFI handler of csrc/enf_xla_ffi.cc does not yet
+request it; differentiate x through enf_pde_b200.nef until it does.
 
 This module needs JAX and the shim library built from csrc/enf_xla_ffi.cc (see its header).  Neither exists in the image
 this repo was developed in (no jax wheel, no network), so this file is exercised only where JAX is installed; everything
@@ -99,7 +101,7 @@ def make_enf_apply(num_hidden, num_heads, num_out, latent_dim, invariant_type, n
         outs = outs[1:]
         n = len(leaves)
         dsigma = outs[n + 2] if use_gaussian_window else None
-        return (list(outs[:n]), jnp.zeros_like(x), outs[n], outs[n + 1], dsigma)
+        return (list(outs[:n]), jnp.zeros_like(x), outs[n], outs[n + 1], dsigma)     # x: see the module docstring
 
     enf_apply.defvjp(vjp_fwd, vjp_bwd)
     return enf_apply

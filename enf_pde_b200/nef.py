@@ -6,8 +6,9 @@ same constructor fields, same argument order `(x, p, a, gaussian_window_size)`, 
 tree (`{'params': {...}}` with Flax's names, SURVEY.md A.3) and the same latent layout
 `p (B,Z,P_raw)`, `a (B,Z,L)`, `gaussian_window (B,Z,1)` (enf/latents/autodecoder.py:58-73).
 PyTorch is used only as plumbing (device memory, streams, autograd tape); all arithmetic of the path
-runs in libenf_b200.so.  The op is ONCE differentiable (first-order gradients w.r.t. parameters,
-p, a and the window size; none w.r.t. the coordinates, which the reference never needs).
+runs in libenf_b200.so.  The op is ONCE differentiable: first-order gradients w.r.t. parameters,
+p, a, the window size and the coordinates x (spatial derivatives of the decoded field; computed only
+when x requires grad, ENF_FLAG_GRAD_X).  For a shared 2-D grid x the gradient is the sum over fields.
 """
 import ctypes
 import math
@@ -76,7 +77,7 @@ def _as_f32(t, name):
 
 
 class _XAttnFunction(torch.autograd.Function):
-    """enf_xattn_fwd / enf_xattn_bwd on torch's current stream."""
+    """enf_xattn_fwd / enf_xattn_bwd (enf_xattn_bwd_x when x needs a gradient) on torch's current stream."""
 
     @staticmethod
     def forward(ctx, meta, x, p, a, sigma, *leaves):
@@ -137,16 +138,21 @@ class _XAttnFunction(torch.autograd.Function):
         dp = torch.empty(ctx.p_shape, dtype=p.dtype, device=p.device) if ctx.n_extra else torch.empty_like(p)
         da = torch.empty_like(a)
         dsigma = torch.empty_like(sigma) if sigma is not None else None
+        # x: [B,C,Dx], or the shared grid [C,Dx] (then dx sums the fields; the caller's expand carries it back)
+        dx = torch.empty_like(x) if ctx.needs_input_grad[1] and desc.flags & _lib.FLAG_GRAD_X else None
         w = _weights_struct(leaves)
         gw = _weights_struct(grads) if need_w else None
         stream = ctypes.c_void_p(torch.cuda.current_stream(x.device).cuda_stream)
         with torch.cuda.device(x.device):
-            rc = lib.enf_xattn_bwd(ctypes.byref(desc), ctypes.byref(w), _ptr(x), ctx.xbs, _ptr(p), _ptr(a), _ptr(sigma),
-                                   _ptr(d_out), ctypes.byref(gw) if need_w else None, _ptr(dp), _ptr(da), _ptr(dsigma),
-                                   _ptr(ctx.ws), ctx.nbytes, stream)
-        _lib.check(rc, "enf_xattn_bwd")
+            args = (ctypes.byref(desc), ctypes.byref(w), _ptr(x), ctx.xbs, _ptr(p), _ptr(a), _ptr(sigma), _ptr(d_out),
+                    ctypes.byref(gw) if need_w else None, _ptr(dp), _ptr(da), _ptr(dsigma))
+            if dx is not None:
+                rc = lib.enf_xattn_bwd_x(*args, _ptr(dx), _ptr(ctx.ws), ctx.nbytes, stream)
+            else:
+                rc = lib.enf_xattn_bwd(*args, _ptr(ctx.ws), ctx.nbytes, stream)
+        _lib.check(rc, "enf_xattn_bwd_x" if dx is not None else "enf_xattn_bwd")
         _XAttnFunction.last_launches[1] = lib.enf_last_launch_count()
-        return (None, None, dp, da, dsigma, *(grads if need_w else [None] * len(leaves)), *([None] * ctx.n_extra))
+        return (None, dx, dp, da, dsigma, *(grads if need_w else [None] * len(leaves)), *([None] * ctx.n_extra))
 
 
 _XAttnFunction.last_launches = [0, 0]
@@ -274,9 +280,11 @@ class EquivariantCrossAttentionNeF:
         sigma = gaussian_window_size if self.use_gaussian_window else None
         if sigma is not None and tuple(sigma.shape) != (B, Z, 1):
             raise ValueError(f"gaussian_window_size must have shape {(B, Z, 1)}")
+        # gradient w.r.t. the coordinates: set at forward time (the workspace then holds the query-record cotangents)
+        grad_x = torch.is_grad_enabled() and x.requires_grad
         desc = dict(B=B, C=C, Z=Z, d=self.num_hidden, H=self.num_heads, L=self.latent_dim, O=self.num_out, Dx=Dx,
                     invariant_kind=_lib.INVARIANT_KINDS[inv.invariant_type], use_window=int(self.use_gaussian_window),
-                    precision=self.precision, flags=0)
+                    precision=self.precision, flags=_lib.FLAG_GRAD_X if grad_x else 0)
         if self.num_layers > 0:
             # latent self-attention steps first (equivariant_cross_attention_nef.py:223-226): a <- gelu(a + block_i(p, p, a)); each is one
             # call of the same C entry points with ENF_FLAG_SELF_BLOCK; the first applies latent_stem, the decode call below none
@@ -303,7 +311,7 @@ class EquivariantCrossAttentionNeF:
             desc["flags"] |= _lib.FLAG_FROZEN_RELU
             return _XAttnFunction.apply((desc, x_shared), x_arg, p, a, sigma, *leaves, relu_mask_pose.detach())
         # forward only (validation roll-outs, pde_trainer.py:389-405): nothing is kept for a backward
-        if not (torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (p, a, sigma, *leaves))):
+        if not (grad_x or torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (p, a, sigma, *leaves))):
             desc["flags"] |= _lib.FLAG_FORWARD_ONLY
             if self.out_bf16:
                 desc["flags"] |= _lib.FLAG_OUT_BF16

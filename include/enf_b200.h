@@ -89,7 +89,13 @@ enum EnfFlags {
   ENF_FLAG_SELF_BLOCK = 32,
   /* `a` is already the hidden latent state [B,Z,d] (the output of a self-attention step): latent_stem is skipped, L must
    * equal d, stem_w / stem_b are unused (may be NULL), da is [B,Z,d]. */
-  ENF_FLAG_NO_STEM = 64
+  ENF_FLAG_NO_STEM = 64,
+  /* Training call that will also want the gradient w.r.t. the query coordinates x (enf_xattn_bwd_x): spatial derivatives of the
+   * decoded field (gradient / Sobolev losses, PDE residuals), or a gradient that flows on into whatever computed x.  Set at
+   * forward time: the workspace then also holds the cotangent of the per-query records, g_xi [B,C,8] (enf_xattn_workspace_bytes
+   * grows by exactly that buffer).  Not with ENF_FLAG_FORWARD_ONLY, nor with ENF_FLAG_SELF_BLOCK (x is ignored there; dp
+   * already carries the poses in both roles). */
+  ENF_FLAG_GRAD_X = 128
 };
 
 enum EnfError {
@@ -201,6 +207,19 @@ int enf_xattn_bwd(const EnfDesc* desc, const EnfWeights* w,
                   const float* d_out, const EnfWeightGrads* dW,
                   float* dp, float* da, float* dsigma,
                   void* workspace, size_t workspace_bytes, enf_stream_t stream);
+
+/* enf_xattn_bwd plus the gradient w.r.t. the query coordinates (the forward must have run with ENF_FLAG_GRAD_X):
+ *   dx     overwritten; [B,C,Dx] when x_batch_stride == C*Dx, [C,Dx] for one shared grid (x_batch_stride == 0): then dx is the
+ *          sum over the B fields.  Required (non-NULL) on a description with ENF_FLAG_GRAD_X; NULL is accepted only without
+ *          that flag (then this is enf_xattn_bwd), a non-NULL dx without it returns ENF_ERR_STATE.
+ * enf_xattn_bwd on an ENF_FLAG_GRAD_X workspace computes everything but dx, at the cost of a backward without the flag.
+ * Like x itself, dx is reached only through the per-query records: the op is once differentiable in x as in everything else. */
+int enf_xattn_bwd_x(const EnfDesc* desc, const EnfWeights* w,
+                    const float* x, int64_t x_batch_stride,
+                    const float* p, const float* a, const float* sigma,
+                    const float* d_out, const EnfWeightGrads* dW,
+                    float* dp, float* da, float* dsigma, float* dx,
+                    void* workspace, size_t workspace_bytes, enf_stream_t stream);
 
 /* Number of kernels of this library enqueued by the last fwd / bwd call of the calling thread. */
 int enf_last_launch_count(void);
