@@ -62,8 +62,8 @@ void leaf_sizes(const EnfDesc& D, int I, size_t* n) {
 }
 
 // the pair kernels' record layout; self-attention steps use get_sa_invariant's variant (Ponita2D: a third invariant)
-EnfRecordLayout record_layout(const EnfDesc& D) {
-  EnfRecordLayout r = enf_record_layout(D.invariant_kind, D.Dx, D.use_window);
+EnfInvariantLayout record_layout(const EnfDesc& D) {
+  EnfInvariantLayout r = enf_record_layout(D.invariant_kind, D.Dx, D.use_window);
   if ((D.flags & ENF_FLAG_SELF_BLOCK) && D.invariant_kind == ENF_INV_PONITA) {
     r.I = 3;
     if (r.win_kind == ENF_WIN_NP) r.win_row = r.I;
@@ -75,12 +75,12 @@ bool tc_fwd_on(const EnfDesc& D) {
   return D.precision == ENF_PREC_BF16 && enf_pairs_fwd_tc_supported(D.d, D.H) && !(D.flags & ENF_FLAG_SELF_BLOCK);
 }
 
-int validate(const EnfDesc* D, EnfRecordLayout* rl) {
+int validate(const EnfDesc* D, EnfInvariantLayout* rl) {
   if (!D) return fail(ENF_ERR_NULL_POINTER, "desc is NULL");
   if (D->B <= 0 || D->C <= 0 || D->Z <= 0 || D->L <= 0 || D->O <= 0) return fail(ENF_ERR_BAD_DESC, "B, C, Z, L, O must be positive");
   if (!(D->d == 16 || D->d == 32 || D->d == 64 || D->d == 128)) return fail(ENF_ERR_UNSUPPORTED, "num_hidden must be 16, 32, 64 or 128");
   if (D->H < 1 || D->H > 4) return fail(ENF_ERR_UNSUPPORTED, "num_heads must be 1..4");
-  EnfRecordLayout r = record_layout(*D);
+  EnfInvariantLayout r = record_layout(*D);
   if (r.I < 0) return fail(ENF_ERR_BAD_DESC, "unknown invariant_kind");
   int k = D->invariant_kind;
   bool dx_ok = (k <= ENF_INV_ABS_POS) ? (D->Dx >= 1 && D->Dx <= 3)
@@ -275,8 +275,7 @@ EnfPairParams pair_params(const EnfDesc& D, const EnfRecordLayout& rl, const Enf
                           const float* sigma, int64_t xi_bs) {
   EnfPairParams p;
   memset(&p, 0, sizeof(p));
-  p.B = D.B; p.C = D.C; p.Z = D.Z; p.H = D.H; p.I = rl.I;
-  p.row_kind = rl.row_kind; p.win_kind = rl.win_kind; p.win_row = rl.win_row; p.nsq = rl.nsq;
+  p.B = D.B; p.C = D.C; p.Z = D.Z; p.H = D.H; p.rec = rl;
   p.xi = c.f("xi"); p.xi_bs = xi_bs; p.lam = c.f("lam"); p.sigma = sigma;
   p.lam_mask = (D.flags & ENF_FLAG_FROZEN_RELU) ? c.f("lam_mask") : nullptr;
   p.q_omega = w.q_omega; p.v_omega = w.v_omega;
@@ -294,8 +293,7 @@ EnfPairTcParams tc_fwd_params(const EnfDesc& D, const EnfRecordLayout& rl, const
                               bool keep_logits, bool stash) {
   EnfPairTcParams tp;
   memset(&tp, 0, sizeof(tp));
-  tp.B = D.B; tp.C = D.C; tp.Z = D.Z; tp.I = rl.I;
-  tp.row_kind = rl.row_kind; tp.win_kind = rl.win_kind; tp.win_row = rl.win_row; tp.nsq = rl.nsq;
+  tp.B = D.B; tp.C = D.C; tp.Z = D.Z; tp.rec = rl;
   tp.xi = pp.xi; tp.xi_bs = pp.xi_bs; tp.lam = pp.lam; tp.sigma = pp.sigma;
   tp.q_omega = w.q_omega; tp.v_omega = w.v_omega; tp.q_b1 = w.q_b1; tp.v_b1 = w.v_b1; tp.bp = c.f("bp");
   tp.img_q_w1 = (const uint8_t*)c.f("img_q_w1"); tp.img_v_w1 = (const uint8_t*)c.f("img_v_w1");
@@ -404,13 +402,13 @@ int enf_debug_gemm(int use_tc, int M, int N, int K, const float* A, int64_t a_rs
 }
 
 size_t enf_xattn_workspace_bytes(const EnfDesc* desc) {
-  EnfRecordLayout rl;
+  EnfInvariantLayout rl;
   if (validate(desc, &rl) != ENF_OK) return 0;
   return make_layout(*desc, rl).total * sizeof(float);
 }
 
 int enf_xattn_chunk_for_cap(const EnfDesc* desc, size_t cap_bytes) {
-  EnfRecordLayout rl;
+  EnfInvariantLayout rl;
   if (validate(desc, &rl) != ENF_OK) return 0;
   EnfDesc D = *desc;
   D.flags |= ENF_FLAG_RECOMPUTE;
@@ -438,7 +436,7 @@ void enf_workspace_release(void* workspace) {
 }
 
 int64_t enf_debug_ws_offset(const EnfDesc* desc, const char* name, int64_t* num_floats) {
-  EnfRecordLayout rl;
+  EnfInvariantLayout rl;
   if (validate(desc, &rl) != ENF_OK || !name) return -1;
   Layout Y = make_layout(*desc, rl);
   for (auto& b : Y.bufs)
@@ -450,7 +448,7 @@ int enf_xattn_fwd(const EnfDesc* desc, const EnfWeights* w, const float* x, int6
                   const float* a, const float* sigma, float* out, void* workspace, size_t workspace_bytes,
                   enf_stream_t stream) {
   g_launches = 0;
-  EnfRecordLayout rl;
+  EnfInvariantLayout rl;
   int rc = validate(desc, &rl);
   if (rc != ENF_OK) return rc;
   const EnfDesc& D = *desc;
@@ -620,7 +618,7 @@ int xattn_bwd(const EnfDesc* desc, const EnfWeights* w, const float* x, int64_t 
               const float* a, const float* sigma, const float* d_out, const EnfWeightGrads* dW, float* dp, float* da,
               float* dsigma, float* dx, bool want_dx, void* workspace, size_t workspace_bytes, enf_stream_t stream) {
   g_launches = 0;
-  EnfRecordLayout rl;
+  EnfInvariantLayout rl;
   int rc = validate(desc, &rl);
   if (rc != ENF_OK) return rc;
   const EnfDesc& D = *desc;
@@ -737,8 +735,7 @@ int xattn_bwd(const EnfDesc* desc, const EnfWeights* w, const float* x, int64_t 
   if (tc_bwd) {
     EnfPairTcBwdParams tp;
     memset(&tp, 0, sizeof(tp));
-    tp.B = D.B; tp.C = D.C; tp.Z = D.Z; tp.I = rl.I;
-    tp.row_kind = rl.row_kind; tp.win_kind = rl.win_kind; tp.win_row = rl.win_row; tp.nsq = rl.nsq;
+    tp.B = D.B; tp.C = D.C; tp.Z = D.Z; tp.rec = rl;
     tp.xi = pp.xi; tp.xi_bs = pp.xi_bs; tp.lam = pp.lam; tp.sigma = pp.sigma;
     tp.q_omega = w->q_omega; tp.v_omega = w->v_omega; tp.q_b1 = w->q_b1; tp.v_b1 = w->v_b1; tp.bp = c.f("bp");
     tp.img_q_w1 = (const uint8_t*)c.f("img_q_w1"); tp.img_v_w1 = (const uint8_t*)c.f("img_v_w1");

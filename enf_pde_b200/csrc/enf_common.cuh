@@ -20,11 +20,12 @@ struct EnfRecordLayout {
   int win_kind;   // ENF_WIN_*
   int win_row;    // row of Lam holding the window's record (== I), or -1 when the window reads u[0]
   int nsq;        // components compared by SQDIST rows
-  int P;          // raw pose width
 };
+// ... and the raw pose width, which only the record producers read (enf_stages.cu)
+struct EnfInvariantLayout : EnfRecordLayout { int P; };
 
-__host__ __device__ inline EnfRecordLayout enf_record_layout(int kind, int Dx, int use_window) {
-  EnfRecordLayout r;
+__host__ __device__ inline EnfInvariantLayout enf_record_layout(int kind, int Dx, int use_window) {
+  EnfInvariantLayout r;
   r.row_kind = ENF_ROW_DOT; r.nsq = Dx; r.win_row = -1;
   int win = ENF_WIN_NP;
   switch (kind) {
@@ -43,6 +44,129 @@ __host__ __device__ inline EnfRecordLayout enf_record_layout(int kind, int Dx, i
   if (r.win_kind == ENF_WIN_NP) r.win_row = r.I;
   if (r.win_kind == ENF_WIN_SPH && kind != ENF_INV_POLAR_PERIODIC) r.win_row = r.I;
   return r;
+}
+
+// ---- the record algebra of one (query, latent) pair, shared by every pair kernel (fp32, tensor-core, latent ODE) ---------
+// lam: the latent's record Lam [ENF_R_LAM][ENF_F_XI]; x / xi: the query's record [ENF_F_XI].  SQDIST rows compare nsq <= 3 components.
+struct EnfPairRecord { float u[6]; float w; float c; };   // invariants, window value, raw cosine (spherical windows)
+
+// invariant row r of one pair: u_r = post(row_r(Lam, xi))
+__device__ __forceinline__ float record_row(const EnfRecordLayout& rl, const float* lam, const float* x, int r) {
+  const float* L = lam + r * ENF_F_XI;
+  float v = 0.f;
+  if (rl.row_kind == ENF_ROW_DOT) {
+#pragma unroll
+    for (int f = 0; f < 8; ++f) v = fmaf(L[f], x[f], v);
+  } else {
+#pragma unroll
+    for (int f = 0; f < 3; ++f) if (f < rl.nsq) { float dl = L[f] - x[f]; v = fmaf(dl, dl, v); }
+    if (rl.row_kind == ENF_ROW_SQDIST_SQRT) v = sqrtf(v);
+  }
+  return v;
+}
+
+// window value w (and the raw cosine c of the spherical windows) from the invariants it reads (u0, u1) and the window row.
+// FAST_EXP: __expf on the tensor-core path (its 16-bit operands dominate the error), expf on the fp32 path (the accurate one).
+template <bool FAST_EXP>
+__device__ __forceinline__ void record_window(const EnfRecordLayout& rl, const float* lam, const float* x, float sigma, float u0, float u1,
+                                              float& w, float& c) {
+  w = 0.f; c = 0.f;
+  if (rl.win_kind == ENF_WIN_NONE) return;
+  const float* L = lam + rl.I * ENF_F_XI;
+  float inv_s2 = 1.f / (sigma * sigma);
+  if (rl.win_kind == ENF_WIN_NP) {
+    float v = 0.f;
+#pragma unroll
+    for (int f = 0; f < 3; ++f) if (f < rl.nsq) { float dl = L[f] - x[f]; v = fmaf(dl, dl, v); }
+    w = -v * inv_s2;
+  } else if (rl.win_kind == ENF_WIN_PER) {
+    w = fmaf(u0, u0, u1 * u1) * inv_s2;
+  } else {
+    c = u0;
+    if (rl.win_row >= 0) {
+      c = 0.f;
+#pragma unroll
+      for (int f = 0; f < 8; ++f) c = fmaf(L[f], x[f], c);
+    }
+    float cl = fminf(fmaxf(c, -1.f + 1e-6f), 1.f - 1e-6f);
+    float ac = acosf(cl);
+    w = FAST_EXP ? __expf(-ac * ac * 0.5f * inv_s2) : expf(-ac * ac * 0.5f * inv_s2);
+  }
+}
+// the invariants u0, u1 that record_window reads, for a caller that holds none of them (0 where the window does not read them)
+__device__ __forceinline__ void record_window_rows(const EnfRecordLayout& rl, const float* lam, const float* x, float& u0, float& u1) {
+  u0 = 0.f; u1 = 0.f;
+  if (rl.win_kind == ENF_WIN_PER) { u0 = record_row(rl, lam, x, 0); u1 = record_row(rl, lam, x, 1); }
+  else if (rl.win_kind == ENF_WIN_SPH && rl.win_row < 0) u0 = record_row(rl, lam, x, 0);
+}
+
+template <bool FAST_EXP>
+__device__ __forceinline__ EnfPairRecord pair_record(const EnfRecordLayout& rl, const float* lam, const float* xi, float sigma) {
+  EnfPairRecord r;
+  float x[8];
+#pragma unroll
+  for (int f = 0; f < 8; ++f) x[f] = xi[f];
+#pragma unroll
+  for (int i = 0; i < 6; ++i) r.u[i] = i < rl.I ? record_row(rl, lam, x, i) : 0.f;
+  record_window<FAST_EXP>(rl, lam, x, sigma, r.u[0], r.u[1], r.w, r.c);
+  return r;
+}
+
+// cotangent of the squared distance v of a SQDIST_SQRT row u = sqrt(v) from the cotangent du of u
+__device__ __forceinline__ float record_sqrt_adjoint(float du, float u) { return u > 0.f ? du / (2.f * u) : 0.f; }
+
+// cotangents of one pair's record rows dq (dq[I]: the window row) and of sigma from those of the invariants (du; the periodic
+// window and the spherical window without a window row add to du[0..1]) and of the window value (dw)
+__device__ __forceinline__ void record_adjoint(const EnfRecordLayout& rl, const EnfPairRecord& rec, float (&du)[6], float dw, float sigma,
+                                               float (&dq)[ENF_R_LAM], float& dsg) {
+#pragma unroll
+  for (int r = 0; r < ENF_R_LAM; ++r) dq[r] = 0.f;
+  dsg = 0.f;
+  if (rl.win_kind != ENF_WIN_NONE) {
+    const float inv_s2 = 1.f / (sigma * sigma);
+    if (rl.win_kind == ENF_WIN_NP) {
+      dq[rl.I] = -dw * inv_s2;
+      dsg = dw * (-2.f * rec.w / sigma);
+    } else if (rl.win_kind == ENF_WIN_PER) {
+      du[0] += dw * 2.f * rec.u[0] * inv_s2;
+      du[1] += dw * 2.f * rec.u[1] * inv_s2;
+      dsg = dw * (-2.f * rec.w / sigma);
+    } else {
+      float cl = fminf(fmaxf(rec.c, -1.f + 1e-6f), 1.f - 1e-6f);
+      float ac = acosf(cl);
+      float dc = (rec.c > -1.f + 1e-6f && rec.c < 1.f - 1e-6f) ? dw * rec.w * ac * inv_s2 * rsqrtf(1.f - cl * cl) : 0.f;
+      if (rl.win_row >= 0) dq[rl.I] = dc; else du[0] += dc;
+      dsg = dw * rec.w * ac * ac * inv_s2 / sigma;
+    }
+  }
+#pragma unroll
+  for (int r = 0; r < 6; ++r) {
+    if (r < rl.I) {
+      if (rl.row_kind == ENF_ROW_SQDIST_SQRT) dq[r] = record_sqrt_adjoint(du[r], rec.u[r]);
+      else dq[r] = du[r];
+    }
+  }
+}
+
+// g[k] += d xi[f] = sum_r dq_r d row_r / d xi[f] for the half f = 4 half + k, k < 4 of the query record: DOT rows are bilinear in
+// (Lam, xi); squared-distance rows (and the non-periodic window row) are sum_{f < nsq} (Lam_f - xi_f)^2, so they only reach half 0
+__device__ __forceinline__ void record_xi_cotangent(const EnfRecordLayout& rl, const float* lam, const float* xi, const float (&dq)[ENF_R_LAM],
+                                                    int half, float* g) {
+  const float* Lh = lam + 4 * half;
+#pragma unroll
+  for (int r = 0; r < ENF_R_LAM; ++r) {
+    if (r < rl.I || (r == rl.I && rl.win_row >= 0)) {
+      const float* L = Lh + r * ENF_F_XI;
+      const bool sq = r < rl.I ? (rl.row_kind != ENF_ROW_DOT) : (rl.win_kind == ENF_WIN_NP);
+      if (!sq) {
+#pragma unroll
+        for (int k = 0; k < 4; ++k) g[k] = fmaf(dq[r], L[k], g[k]);
+      } else if (half == 0) {
+#pragma unroll
+        for (int k = 0; k < 3; ++k) if (k < rl.nsq) g[k] = fmaf(-2.f * dq[r], L[k] - xi[k], g[k]);
+      }
+    }
+  }
 }
 
 // jax.nn.gelu(approximate=True)
@@ -153,8 +277,8 @@ int enf_launch_weight_image_T(cudaStream_t st, const float* W, void* img, int N,
 
 // ---- fused pair kernels (enf_pairs_simt.cu) ------------------------------------------------------
 struct EnfPairParams {
-  int B, C, Z, H, I;
-  int row_kind, win_kind, win_row, nsq;
+  int B, C, Z, H;
+  EnfRecordLayout rec;
   const float* xi;  int64_t xi_bs;           // [Bx, C, 8]
   const float* lam;                          // [B, Z, 7, 8]
   const float* lam_mask;                     // frozen-relu mode (ENF_FLAG_FROZEN_RELU): record of the mask poses, else null
@@ -179,8 +303,8 @@ int enf_launch_pairs_bwd_simt(cudaStream_t st, int d, const EnfPairParams& p);
 
 // ---- tensor-core pair kernels (enf_pairs_tc.cu) ----------------------------------------------------
 struct EnfPairTcParams {
-  int B, C, Z, I;
-  int row_kind, win_kind, win_row, nsq;
+  int B, C, Z;
+  EnfRecordLayout rec;
   const float* xi;  int64_t xi_bs;
   const float* lam; const float* sigma;
   const float* q_omega; const float* v_omega;
@@ -200,8 +324,8 @@ int enf_launch_pairs_fwd_tc(cudaStream_t st, int d, int H, const EnfPairTcParams
 
 struct __half;
 struct EnfPairTcBwdParams {
-  int B, C, Z, I;
-  int row_kind, win_kind, win_row, nsq;
+  int B, C, Z;
+  EnfRecordLayout rec;
   const float* xi;  int64_t xi_bs;
   const float* lam; const float* sigma;
   const float* q_omega; const float* v_omega;

@@ -20,7 +20,8 @@ namespace {
 
 struct Dims {
   int B, Z, L, Hd, Bd, NL, W, deg, Dx, kind;
-  int I, P, npos, nori, S, F, Fp, row_kind, nsq;      // Fp: row stride of the feature matrices (F rounded up to 32)
+  EnfInvariantLayout rec;                            // of the pair invariants (rec.I: their width, rec.P: the pose width)
+  int npos, nori, S, F, Fp;                         // Fp: row stride of the feature matrices (F rounded up to 32)
   int64_t m, n;
 };
 
@@ -31,7 +32,7 @@ int validate(const EnfOdeDesc* D, Dims* o) {
   if (D->layers < 1 || D->layers > ENF_ODE_MAX_LAYERS) return enf_set_error(ENF_ERR_UNSUPPORTED, "layers must be 1..ENF_ODE_MAX_LAYERS");
   if (D->degree < 0 || D->degree > 5) return enf_set_error(ENF_ERR_UNSUPPORTED, "degree must be 0..5");
   for (int i = 0; i < 6; ++i) if (D->reserved[i]) return enf_set_error(ENF_ERR_BAD_DESC, "reserved fields must be 0");
-  EnfRecordLayout r = enf_record_layout(D->invariant_kind, D->Dx, 0);
+  EnfInvariantLayout r = enf_record_layout(D->invariant_kind, D->Dx, 0);
   if (r.I < 0) return enf_set_error(ENF_ERR_BAD_DESC, "unknown invariant_kind");
   const int k = D->invariant_kind;
   const bool dx_ok = (k == ENF_INV_REL_POS || k == ENF_INV_NORM_REL_POS || k == ENF_INV_ABS_POS) ? (D->Dx >= 1 && D->Dx <= 3)
@@ -40,11 +41,12 @@ int validate(const EnfOdeDesc* D, Dims* o) {
   Dims d;
   d.B = D->B; d.Z = D->Z; d.L = D->L; d.Hd = D->hidden; d.Bd = D->basis; d.NL = D->layers; d.W = D->widen * D->hidden;
   d.deg = D->degree; d.Dx = D->Dx; d.kind = k;
-  d.I = k == ENF_INV_PONITA ? 3 : r.I;            // Ponita2D (get_sa_invariant), ponita.py:46-86
-  d.P = r.P; d.nori = k == ENF_INV_PONITA ? 1 : 0; d.npos = d.P - d.nori;
-  d.S = d.L + d.nori; d.row_kind = r.row_kind; d.nsq = r.nsq;
+  d.rec = r;
+  if (k == ENF_INV_PONITA) d.rec.I = 3;           // Ponita2D (get_sa_invariant), ponita.py:46-86
+  d.nori = k == ENF_INV_PONITA ? 1 : 0; d.npos = d.rec.P - d.nori;
+  d.S = d.L + d.nori;
   int64_t F = 0, pw = 1;
-  for (int t = 0; t <= d.deg; ++t) { pw *= d.I; F += pw; }
+  for (int t = 0; t <= d.deg; ++t) { pw *= d.rec.I; F += pw; }
   if (F > 4096) return enf_set_error(ENF_ERR_UNSUPPORTED, "tensor-power feature width above 4096");
   d.F = (int)F;
   d.Fp = (d.F + 31) / 32 * 32;
@@ -74,7 +76,7 @@ struct Ws {
 Ws make_ws(const Dims& d) {
   Ws w;
   w.lam = w.take(d.m * ENF_LAM_SIZE); w.xi = w.take(d.m * ENF_F_XI);
-  w.inv = w.take(d.n * d.I); w.poly = w.take(d.n * d.Fp);
+  w.inv = w.take(d.n * d.rec.I); w.poly = w.take(d.n * d.Fp);
   w.h0p = w.take(d.n * d.Hd); w.h0 = w.take(d.n * d.Hd); w.kbp = w.take(d.n * d.Bd); w.kb = w.take(d.n * d.Bd);
   w.am1 = w.take(d.m * d.L);
   for (int l = 0; l <= d.NL; ++l) w.hin[l] = w.take(d.m * d.Hd);
@@ -87,29 +89,17 @@ Ws make_ws(const Dims& d) {
   for (int l = 0; l < d.NL; ++l) w.cklo[l] = w.take((int64_t)d.Bd * d.Hd);
   w.g_scalar = w.take(d.m * d.S); w.g_ha = w.take(d.m * d.Hd); w.g_hb = w.take(d.m * d.Hd); w.g_l1 = w.take(d.m * d.W);
   w.g_ln = w.take(d.m * d.Hd); w.g_c = w.take(d.m * d.Hd); w.g_K = w.take(d.n * d.Hd); w.g_kb = w.take(d.n * d.Bd);
-  w.g_kbp = w.take(d.n * d.Bd); w.g_h0 = w.take(d.n * d.Hd); w.g_poly = w.take(d.n * d.Fp); w.g_inv = w.take(d.n * d.I);
+  w.g_kbp = w.take(d.n * d.Bd); w.g_h0 = w.take(d.n * d.Hd); w.g_poly = w.take(d.n * d.Fp); w.g_inv = w.take(d.n * d.rec.I);
   w.gw = w.take(d.n * 2); w.g_lam = w.take(d.m * ENF_LAM_SIZE); w.g_xi = w.take(d.m * ENF_F_XI); w.ssum = w.take(d.m * 2);
-  w.gpe = w.take(d.m * 8); w.rosum = w.take(2 * (d.I + d.Hd));
-  for (int i = 0; i < 4; ++i) { w.kp[i] = w.take(d.m * d.P); w.ka[i] = w.take(d.m * d.L); }
-  w.tp = w.take(d.m * d.P); w.ta = w.take(d.m * d.L); w.sp = w.take(d.m * d.P); w.sa = w.take(d.m * d.L);
+  w.gpe = w.take(d.m * 8); w.rosum = w.take(2 * (d.rec.I + d.Hd));
+  for (int i = 0; i < 4; ++i) { w.kp[i] = w.take(d.m * d.rec.P); w.ka[i] = w.take(d.m * d.L); }
+  w.tp = w.take(d.m * d.rec.P); w.ta = w.take(d.m * d.L); w.sp = w.take(d.m * d.rec.P); w.sa = w.take(d.m * d.L);
   return w;
 }
 
 inline int nblocks(int64_t n, int per) { return (int)((n + per - 1) / per); }
 
 // ---- kernels ------------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ float ode_inv_row(int row_kind, int nsq, const float* L, const float* x) {
-  float v = 0.f;
-  if (row_kind == ENF_ROW_DOT) {
-#pragma unroll
-    for (int f = 0; f < 8; ++f) v = fmaf(L[f], x[f], v);
-  } else {
-    for (int f = 0; f < nsq; ++f) { float dl = L[f] - x[f]; v = fmaf(dl, dl, v); }
-    if (row_kind == ENF_ROW_SQDIST_SQRT) v = sqrtf(v);
-  }
-  return v;
-}
-
 __global__ void ode_am1_kernel(const float* __restrict__ a, float* __restrict__ am1, int64_t total) {      // ponita_ode_g.py:233
   int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (t < total) am1[t] = a[t] - 1.f;
@@ -136,7 +126,7 @@ __global__ void ode_poly_table_kernel(int I, int F, uint32_t* __restrict__ tab) 
 
 // invariants of every pair row and their tensor powers [u, u (x) u, ...].  One warp per pair row; lanes stride over the F
 // features (coalesced stores).
-__global__ void __launch_bounds__(256) ode_inv_poly_kernel(int I, int F, int Fp, int row_kind, int nsq, int Z, int64_t n,
+__global__ void __launch_bounds__(256) ode_inv_poly_kernel(EnfRecordLayout rl, int F, int Fp, int Z, int64_t n,
                                                            const float* __restrict__ lam, const float* __restrict__ xi,
                                                            const uint32_t* __restrict__ tab, float* __restrict__ inv,
                                                            float* __restrict__ poly) {
@@ -146,10 +136,10 @@ __global__ void __launch_bounds__(256) ode_inv_poly_kernel(int I, int F, int Fp,
   if (row >= n) return;
   const int64_t br = row / Z;                    // (b, r)
   const int64_t bs = (br / Z) * Z + row % Z;     // (b, s)
-  if (lane < I) {
-    float u = ode_inv_row(row_kind, nsq, lam + bs * ENF_LAM_SIZE + lane * ENF_F_XI, xi + br * ENF_F_XI);
+  if (lane < rl.I) {
+    float u = record_row(rl, lam + bs * ENF_LAM_SIZE, xi + br * ENF_F_XI, lane);
     su[wl][lane] = u;
-    inv[row * I + lane] = u;
+    inv[row * rl.I + lane] = u;
   }
   __syncwarp();
   const float* u = su[wl];
@@ -387,28 +377,24 @@ __global__ void ode_readout_bwd_h_kernel(int I, int Hd, int64_t m, const float* 
   if (rosum) { atomicAdd(rosum + I + c, ar); if (ro_ori) atomicAdd(rosum + I + Hd + I + c, ao); }
 }
 
-// cotangent of the squared distance from the cotangent of a SQDIST(_SQRT) row
-__device__ __forceinline__ float ode_dq(int row_kind, float du, float u) {
-  if (row_kind == ENF_ROW_SQDIST_SQRT) return u > 0.f ? du / (2.f * u) : 0.f;
-  return du;
-}
 // g_lam[bs][i][f] = sum_r dq[(b,r,s)][i] xi[(b,r)][f]   (what the ENF pair backward accumulates per latent, enf_stages.cu)
-__global__ void ode_inv_bwd_lam_kernel(int I, int Z, int row_kind, int64_t total, const float* __restrict__ inv,
+__global__ void ode_inv_bwd_lam_kernel(EnfRecordLayout rl, int Z, int64_t total, const float* __restrict__ inv,
                                        const float* __restrict__ g_inv, const float* __restrict__ xi, float* __restrict__ g_lam) {
   int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= total) return;
   const int f = (int)(t % ENF_F_XI), i = (int)((t / ENF_F_XI) % ENF_R_LAM);
   const int64_t bs = t / ENF_LAM_SIZE, b = bs / Z, s = bs % Z;
   float acc = 0.f;
-  if (i < I)
+  if (i < rl.I)
     for (int r = 0; r < Z; ++r) {
       const int64_t br = b * Z + r, row = br * Z + s;
-      acc = fmaf(ode_dq(row_kind, g_inv[row * I + i], inv[row * I + i]), xi[br * ENF_F_XI + f], acc);
+      const float du = g_inv[row * rl.I + i];
+      acc = fmaf(rl.row_kind == ENF_ROW_SQDIST_SQRT ? record_sqrt_adjoint(du, inv[row * rl.I + i]) : du, xi[br * ENF_F_XI + f], acc);
     }
   g_lam[t] = acc;
 }
 // g_xi[br][f] = sum_s sum_i du Lam[(b,s)][i][f]  (DOT rows)  |  sum_s -2 dq (Lam[(b,s)][0][f] - xi[br][f])  (SQDIST rows, f < nsq)
-__global__ void ode_inv_bwd_xi_kernel(int I, int Z, int row_kind, int nsq, int64_t total, const float* __restrict__ inv,
+__global__ void ode_inv_bwd_xi_kernel(EnfRecordLayout rl, int Z, int64_t total, const float* __restrict__ inv,
                                       const float* __restrict__ g_inv, const float* __restrict__ lam, const float* __restrict__ xi,
                                       float* __restrict__ g_xi) {
   int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -416,17 +402,19 @@ __global__ void ode_inv_bwd_xi_kernel(int I, int Z, int row_kind, int nsq, int64
   const int f = (int)(t % ENF_F_XI);
   const int64_t br = t / ENF_F_XI, b = br / Z;
   float acc = 0.f;
-  if (row_kind == ENF_ROW_DOT) {
+  if (rl.row_kind == ENF_ROW_DOT) {
     for (int s = 0; s < Z; ++s) {
       const int64_t row = br * Z + s;
       const float* Lm = lam + (b * Z + s) * ENF_LAM_SIZE + f;
-      for (int i = 0; i < I; ++i) acc = fmaf(g_inv[row * I + i], Lm[i * ENF_F_XI], acc);
+      for (int i = 0; i < rl.I; ++i) acc = fmaf(g_inv[row * rl.I + i], Lm[i * ENF_F_XI], acc);
     }
-  } else if (f < nsq) {
+  } else if (f < rl.nsq) {
     const float x = xi[br * ENF_F_XI + f];
     for (int s = 0; s < Z; ++s) {
       const int64_t row = br * Z + s;
-      acc = fmaf(-2.f * ode_dq(row_kind, g_inv[row * I], inv[row * I]), lam[(b * Z + s) * ENF_LAM_SIZE + f] - x, acc);
+      const float du = g_inv[row * rl.I];
+      const float dq = rl.row_kind == ENF_ROW_SQDIST_SQRT ? record_sqrt_adjoint(du, inv[row * rl.I]) : du;
+      acc = fmaf(-2.f * dq, lam[(b * Z + s) * ENF_LAM_SIZE + f] - x, acc);
     }
   }
   g_xi[t] = acc;
@@ -505,11 +493,11 @@ int check_ptrs(const Dims& d, const EnfOdeWeights* w, const void* workspace) {
 int forward(const Dims& d, const Ws& Y, const EnfOdeWeights& w, const float* p, const float* a, float* dp_dt, float* da_dt, Run& R) {
   cudaStream_t st = R.st;
   float* W = R.ws;
-  R.launches += enf_launch_pose_record(st, d.kind, d.Dx, d.P, d.I, d.m, p, W + Y.lam);
-  R.launches += enf_launch_pose_features(st, d.kind, d.Dx, d.P, d.m, p, W + Y.xi);
+  R.launches += enf_launch_pose_record(st, d.kind, d.Dx, d.rec.P, d.rec.I, d.m, p, W + Y.lam);
+  R.launches += enf_launch_pose_features(st, d.kind, d.Dx, d.rec.P, d.m, p, W + Y.xi);
   uint32_t* ptab = reinterpret_cast<uint32_t*>(W + Y.ptab);
-  ode_poly_table_kernel<<<nblocks(d.F, 128), 128, 0, st>>>(d.I, d.F, ptab);
-  ode_inv_poly_kernel<<<nblocks(d.n, 8), 256, 0, st>>>(d.I, d.F, d.Fp, d.row_kind, d.nsq, d.Z, d.n, W + Y.lam, W + Y.xi, ptab, W + Y.inv, W + Y.poly);
+  ode_poly_table_kernel<<<nblocks(d.F, 128), 128, 0, st>>>(d.rec.I, d.F, ptab);
+  ode_inv_poly_kernel<<<nblocks(d.n, 8), 256, 0, st>>>(d.rec, d.F, d.Fp, d.Z, d.n, W + Y.lam, W + Y.xi, ptab, W + Y.inv, W + Y.poly);
   // The pair-row Dense layers run on the tf32 tensor-core kernels as 3-term split products (fp32-level accuracy,
   // enf_gemm_tc.cu) when the shapes allow (hidden, basis multiples of 32, >= 128 pair rows), else on the fp32 kernel: the
   // low parts W - trunc_tf32(W) of the weights they multiply by, and kb_w0 zero-padded to whole 32-feature blocks
@@ -541,8 +529,8 @@ int forward(const Dims& d, const Ws& Y, const EnfOdeWeights& w, const float* p, 
   }
   const float* h = W + Y.hin[d.NL];
   R.gemm(d.m, d.S, d.Hd, enf_mat(h, d.Hd), enf_mat(w.ro_scalar, d.S), enf_mat(W + Y.scalar, d.S));
-  ode_hs_kernel<<<nblocks(d.m, 8), 256, 0, st>>>(d.I, d.Hd, d.m, h, w.ro_rel, d.nori ? w.ro_ori : nullptr, W + Y.hs);
-  ode_readout_fwd_kernel<<<nblocks(d.m, 8), 256, 0, st>>>(d.I, d.Z, d.P, d.npos, d.nori, d.L, d.S, d.m, p, W + Y.inv, W + Y.hs,
+  ode_hs_kernel<<<nblocks(d.m, 8), 256, 0, st>>>(d.rec.I, d.Hd, d.m, h, w.ro_rel, d.nori ? w.ro_ori : nullptr, W + Y.hs);
+  ode_readout_fwd_kernel<<<nblocks(d.m, 8), 256, 0, st>>>(d.rec.I, d.Z, d.rec.P, d.npos, d.nori, d.L, d.S, d.m, p, W + Y.inv, W + Y.hs,
                                                            W + Y.scalar, w.ro_rel, d.nori ? w.ro_ori : nullptr, W + Y.wpair, dp_dt, da_dt);
   R.launches += 6 + 1 * d.NL;
   if (R.failed) return enf_set_error(ENF_ERR_CUDA, "a stage GEMM of the latent ODE model could not be configured");
@@ -600,16 +588,16 @@ int enf_ode_bwd(const EnfOdeDesc* desc, const EnfOdeWeights* w, const float* p, 
       zero(g.conv_k, (int64_t)d.Bd * d.Hd); zero(g.conv_b, d.Hd); zero(g.ln_g, d.Hd); zero(g.ln_b, d.Hd);
       zero(g.l1_w, (int64_t)d.Hd * d.W); zero(g.l1_b, d.W); zero(g.l2_w, (int64_t)d.W * d.Hd); zero(g.l2_b, d.Hd);
     }
-    zero(W + Y.rosum, 2 * (d.I + d.Hd));
+    zero(W + Y.rosum, 2 * (d.rec.I + d.Hd));
   }
   const float* ro_ori = d.nori ? w->ro_ori : nullptr;
   float* rosum = wg ? W + Y.rosum : nullptr;
   const float* h = W + Y.hin[d.NL];
   // ---- read-outs ------------------------------------------------------------------------------------------------------------
-  ode_readout_bwd_r_kernel<<<nblocks(d.m, 8), 256, 0, st>>>(d.I, d.Hd, d.Z, d.P, d.npos, d.nori, d.L, d.S, d.m, p, W + Y.inv, W + Y.wpair,
+  ode_readout_bwd_r_kernel<<<nblocks(d.m, 8), 256, 0, st>>>(d.rec.I, d.Hd, d.Z, d.rec.P, d.npos, d.nori, d.L, d.S, d.m, p, W + Y.inv, W + Y.wpair,
                                                              g_dp, g_da, w->ro_rel, ro_ori, W + Y.gw, W + Y.g_inv, W + Y.gpe, rosum,
                                                              W + Y.g_scalar);
-  ode_readout_bwd_s_kernel<<<nblocks(d.m, 8), 256, 0, st>>>(d.Z, d.P, d.npos, d.nori, d.m, p, W + Y.wpair, W + Y.gw, g_dp, W + Y.ssum, W + Y.gpe);
+  ode_readout_bwd_s_kernel<<<nblocks(d.m, 8), 256, 0, st>>>(d.Z, d.rec.P, d.npos, d.nori, d.m, p, W + Y.wpair, W + Y.gw, g_dp, W + Y.ssum, W + Y.gpe);
   float* g_h = W + Y.g_ha;
   float* g_h2 = W + Y.g_hb;
   R.gemm(d.m, d.Hd, d.S, enf_mat(W + Y.g_scalar, d.S), enf_mat(w->ro_scalar, 1, d.S), enf_mat(g_h, d.Hd));
@@ -617,9 +605,9 @@ int enf_ode_bwd(const EnfOdeDesc* desc, const EnfOdeWeights* w, const float* p, 
   {
     int gx = (int)((d.m + 63) / 64); if (gx > 592) gx = 592;
     dim3 grid(gx, (d.Hd + 127) / 128);
-    ode_readout_bwd_h_kernel<<<grid, 128, 0, st>>>(d.I, d.Hd, d.m, W + Y.ssum, h, w->ro_rel, ro_ori, g_h, rosum);
+    ode_readout_bwd_h_kernel<<<grid, 128, 0, st>>>(d.rec.I, d.Hd, d.m, W + Y.ssum, h, w->ro_rel, ro_ori, g_h, rosum);
   }
-  if (wg) ode_ro_scatter_kernel<<<nblocks(d.I + d.Hd, 128), 128, 0, st>>>(d.I + d.Hd, W + Y.rosum, dW->ro_rel, d.nori ? dW->ro_ori : nullptr);
+  if (wg) ode_ro_scatter_kernel<<<nblocks(d.rec.I + d.Hd, 128), 128, 0, st>>>(d.rec.I + d.Hd, W + Y.rosum, dW->ro_rel, d.nori ? dW->ro_ori : nullptr);
   // ---- interaction layers, last to first; g_kb accumulates the kernel-basis cotangent over the layers -------------------------
   for (int l = d.NL - 1; l >= 0; --l) {
     const EnfOdeLayer& y = w->layer[l];
@@ -673,15 +661,15 @@ int enf_ode_bwd(const EnfOdeDesc* desc, const EnfOdeWeights* w, const float* p, 
     R.gemm(d.n, nc, d.Hd, enf_mat(W + Y.g_h0, d.Hd), enf_mat(W + Y.w0p + (int64_t)c0 * d.Hd, 1, d.Hd), enf_mat(W + Y.g_poly + c0, d.Fp),
            o_tc(EnfGemmOpts(), W + Y.w0lo + (int64_t)c0 * d.Hd));
   }
-  ode_poly_bwd_kernel<<<nblocks(d.n, 8), 256, 0, st>>>(d.I, d.F, d.Fp, d.n, W + Y.inv, W + Y.g_poly, reinterpret_cast<const uint32_t*>(W + Y.ptab), W + Y.g_inv);
+  ode_poly_bwd_kernel<<<nblocks(d.n, 8), 256, 0, st>>>(d.rec.I, d.F, d.Fp, d.n, W + Y.inv, W + Y.g_poly, reinterpret_cast<const uint32_t*>(W + Y.ptab), W + Y.g_inv);
   // ---- invariants -> poses (sender side through Lam, receiver side through xi), read-out position terms ------------------------
-  ode_inv_bwd_lam_kernel<<<nblocks(d.m * ENF_LAM_SIZE, 256), 256, 0, st>>>(d.I, d.Z, d.row_kind, d.m * ENF_LAM_SIZE, W + Y.inv, W + Y.g_inv,
+  ode_inv_bwd_lam_kernel<<<nblocks(d.m * ENF_LAM_SIZE, 256), 256, 0, st>>>(d.rec, d.Z, d.m * ENF_LAM_SIZE, W + Y.inv, W + Y.g_inv,
                                                                            W + Y.xi, W + Y.g_lam);
-  ode_inv_bwd_xi_kernel<<<nblocks(d.m * ENF_F_XI, 256), 256, 0, st>>>(d.I, d.Z, d.row_kind, d.nsq, d.m * ENF_F_XI, W + Y.inv, W + Y.g_inv,
+  ode_inv_bwd_xi_kernel<<<nblocks(d.m * ENF_F_XI, 256), 256, 0, st>>>(d.rec, d.Z, d.m * ENF_F_XI, W + Y.inv, W + Y.g_inv,
                                                                       W + Y.lam, W + Y.xi, W + Y.g_xi);
-  R.launches += enf_launch_pose_record_bwd(st, d.kind, d.Dx, d.P, d.I, ENF_WIN_NONE, d.m, p, W + Y.g_lam, gp);
-  R.launches += enf_launch_pose_features_bwd(st, d.kind, d.Dx, d.P, d.m, p, W + Y.g_xi, gp);
-  ode_add_gpe_kernel<<<nblocks(d.m, 256), 256, 0, st>>>(d.P, d.npos, d.nori, d.m, W + Y.gpe, gp);
+  R.launches += enf_launch_pose_record_bwd(st, d.kind, d.Dx, d.rec.P, d.rec.I, ENF_WIN_NONE, d.m, p, W + Y.g_lam, gp);
+  R.launches += enf_launch_pose_features_bwd(st, d.kind, d.Dx, d.rec.P, d.m, p, W + Y.g_xi, gp);
+  ode_add_gpe_kernel<<<nblocks(d.m, 256), 256, 0, st>>>(d.rec.P, d.npos, d.nori, d.m, W + Y.gpe, gp);
   R.launches += 8;
   if (R.failed) return enf_set_error(ENF_ERR_CUDA, "a stage GEMM of the latent ODE backward could not be configured");
   cudaError_t e = cudaGetLastError();
@@ -704,9 +692,9 @@ int enf_ode_solve(const EnfOdeDesc* desc, const EnfOdeWeights* w, const float* p
   cudaStream_t st = R.st;
   float* W = R.ws;
   const int T1 = num_steps + 1;
-  const int64_t np = d.m * d.P, na = d.m * d.L;
+  const int64_t np = d.m * d.rec.P, na = d.m * d.L;
   auto store = [&](int step, const float* p, const float* a) {
-    ode_store_traj_kernel<<<nblocks(np, 256), 256, 0, st>>>(d.Z, d.P, T1, step, np, p, p_traj);
+    ode_store_traj_kernel<<<nblocks(np, 256), 256, 0, st>>>(d.Z, d.rec.P, T1, step, np, p, p_traj);
     ode_store_traj_kernel<<<nblocks(na, 256), 256, 0, st>>>(d.Z, d.L, T1, step, na, a, a_traj);
   };
   auto axpy = [&](int64_t n, const float* x, float c0, const float* k0, float c1, const float* k1, float c2, const float* k2, float c3,

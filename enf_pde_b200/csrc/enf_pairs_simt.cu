@@ -177,67 +177,6 @@ template <int D> constexpr int small_floats() {
   return TM * 8 * 4 + TM * 3 + MAXH * TM * 5 + 64 + 8 + MAXH * D + 12 * (D / 2) + 64 + TM * 8;
 }
 
-// invariants u[I] and window w of row t against the staged latent record
-__device__ __forceinline__ void pair_invariants(const EnfPairParams& P, const Smem& S, int t, float sigma) {
-  const float* xi = S.xi + t * 8;
-  float q[ENF_R_LAM];
-  const int I = P.I;
-  for (int r = 0; r < I; ++r) {
-    const float* L = S.lam + r * ENF_F_XI;
-    float v = 0.f;
-    if (P.row_kind == ENF_ROW_DOT) {
-#pragma unroll
-      for (int f = 0; f < ENF_F_XI; ++f) v = fmaf(L[f], xi[f], v);
-    } else {
-      for (int i = 0; i < P.nsq; ++i) { float dlt = L[i] - xi[i]; v = fmaf(dlt, dlt, v); }
-      if (P.row_kind == ENF_ROW_SQDIST_SQRT) v = sqrtf(v);
-    }
-    q[r] = v;
-    S.u[t * 8 + r] = v;
-  }
-  float w = 0.f;
-  if (P.win_kind != ENF_WIN_NONE) {
-    const float* L = S.lam + P.I * ENF_F_XI;
-    float inv_s2 = 1.f / (sigma * sigma);
-    if (P.win_kind == ENF_WIN_NP) {
-      float v = 0.f;
-      for (int i = 0; i < P.nsq; ++i) { float dlt = L[i] - xi[i]; v = fmaf(dlt, dlt, v); }
-      w = -v * inv_s2;
-    } else if (P.win_kind == ENF_WIN_PER) {
-      w = (q[0] * q[0] + q[1] * q[1]) * inv_s2;
-    } else {
-      float c = q[0];
-      if (P.win_row >= 0) {
-        c = 0.f;
-#pragma unroll
-        for (int f = 0; f < ENF_F_XI; ++f) c = fmaf(L[f], xi[f], c);
-      }
-      float cl = fminf(fmaxf(c, -1.f + 1e-6f), 1.f - 1e-6f);
-      float ac = acosf(cl);
-      w = expf(-ac * ac * 0.5f * inv_s2);
-      S.u[t * 8 + 7] = c;      // keep the raw cosine for the backward (I <= 6 so slot 7 is free)
-    }
-  }
-  S.w[t] = w;
-}
-
-// invariants only, of row t against record `lam` -> u[t][0..I)   (frozen-relu mode: the mask poses' invariants)
-__device__ __forceinline__ void pair_invariants_only(const EnfPairParams& P, const float* xi_all, const float* lam, float* u, int t) {
-  const float* xi = xi_all + t * 8;
-  for (int r = 0; r < P.I; ++r) {
-    const float* L = lam + r * ENF_F_XI;
-    float v = 0.f;
-    if (P.row_kind == ENF_ROW_DOT) {
-#pragma unroll
-      for (int f = 0; f < ENF_F_XI; ++f) v = fmaf(L[f], xi[f], v);
-    } else {
-      for (int i = 0; i < P.nsq; ++i) { float dlt = L[i] - xi[i]; v = fmaf(dlt, dlt, v); }
-      if (P.row_kind == ENF_ROW_SQDIST_SQRT) v = sqrtf(v);
-    }
-    u[t * 8 + r] = v;
-  }
-}
-
 // gamma(u) = [sin(2 pi u Omega) | cos(2 pi u Omega)]  (rff.py:84-93) into G[TM][D]
 template <int D>
 __device__ __forceinline__ void rff_features(const float* u, const float* om, int I, float* G) {
@@ -294,16 +233,25 @@ __device__ __forceinline__ void pair_chain_common(const EnfPairParams& P, const 
   if (frozen && tid < ENF_LAM_SIZE) S.lam2[tid] = P.lam_mask[bz * ENF_LAM_SIZE + tid];
   __syncthreads();
   if (tid < TM) {
-    pair_invariants(P, S, tid, P.sigma ? P.sigma[bz] : 1.f);
-    if (frozen) pair_invariants_only(P, S.xi, S.lam2, S.u2, tid);
+    const float* xi = S.xi + tid * 8;
+    const EnfPairRecord rec = pair_record<false>(P.rec, S.lam, xi, P.sigma ? P.sigma[bz] : 1.f);
+#pragma unroll
+    for (int r = 0; r < 6; ++r) {
+      if (r < P.rec.I) {
+        S.u[tid * 8 + r] = rec.u[r];
+        if (frozen) S.u2[tid * 8 + r] = record_row(P.rec, S.lam2, xi, r);
+      }
+    }
+    S.u[tid * 8 + 7] = rec.c;      // the raw cosine of a spherical window, for the backward (I <= 6 so slot 7 is free)
+    S.w[tid] = rec.w;
   }
   __syncthreads();
   if (frozen) {
-    rff_features<D>(S.u2, S.omq, P.I, tmpG);
+    rff_features<D>(S.u2, S.omq, P.rec.I, tmpG);
     __syncthreads();
     tile_gemm<D, 0, false>(tmpG, P.q_w1, MQ, P.q_b1, nullptr, Ws);            // pre-activations at the mask poses
   }
-  rff_features<D>(S.u, S.omq, P.I, Gq);
+  rff_features<D>(S.u, S.omq, P.rec.I, Gq);
   __syncthreads();
   if (frozen) tile_gemm<D, 2, false>(Gq, P.q_w1, H1q, P.q_b1, MQ, Ws);
   else tile_gemm<D, 1, false>(Gq, P.q_w1, H1q, P.q_b1, nullptr, Ws);
@@ -317,11 +265,11 @@ __device__ __forceinline__ void pair_chain_common(const EnfPairParams& P, const 
   }
   if (!KEEP) __syncthreads();     // forward aliases Gq/Gv: everyone must be done reading H1q before it is reused
   if (frozen) {
-    rff_features<D>(S.u2, S.omv, P.I, tmpG);
+    rff_features<D>(S.u2, S.omv, P.rec.I, tmpG);
     __syncthreads();
     tile_gemm<D, 0, false>(tmpG, P.v_w1, MV, P.v_b1, nullptr, Ws);
   }
-  rff_features<D>(S.u, S.omv, P.I, Gv);
+  rff_features<D>(S.u, S.omv, P.rec.I, Gv);
   __syncthreads();
   if (frozen) tile_gemm<D, 2, false>(Gv, P.v_w1, H1v, P.v_b1, MV, Ws);
   else tile_gemm<D, 1, false>(Gv, P.v_w1, H1v, P.v_b1, nullptr, Ws);
@@ -358,7 +306,7 @@ __global__ void __launch_bounds__(NT, 1) pairs_fwd_kernel(EnfPairParams P) {
     int row = e >> 3;
     S.xi[e] = row < nv ? P.xi[(int64_t)b * P.xi_bs + (int64_t)(c0 + row) * 8 + (e & 7)] : 0.f;
   }
-  for (int e = tid; e < P.I * (D / 2); e += NT) { S.omq[e] = P.q_omega[e]; S.omv[e] = P.v_omega[e]; }
+  for (int e = tid; e < P.rec.I * (D / 2); e += NT) { S.omq[e] = P.q_omega[e]; S.omv[e] = P.v_omega[e]; }
   for (int e = tid; e < MAXH * TM; e += NT) { S.m[e] = -INFINITY; S.l[e] = 0.f; }
   for (int e = tid; e < H * C::BUF; e += NT) acc[e] = 0.f;
   __syncthreads();
@@ -432,7 +380,7 @@ __global__ void __launch_bounds__(NT, 1) pairs_bwd_kernel(EnfPairParams P) {
     int row = e >> 3;
     S.xi[e] = row < nv ? P.xi[(int64_t)b * P.xi_bs + (int64_t)(c0 + row) * 8 + (e & 7)] : 0.f;
   }
-  for (int e = tid; e < P.I * HD; e += NT) { S.omq[e] = P.q_omega[e]; S.omv[e] = P.v_omega[e]; }
+  for (int e = tid; e < P.rec.I * HD; e += NT) { S.omq[e] = P.q_omega[e]; S.omv[e] = P.v_omega[e]; }
   // lse (kept in S.m) and D = dnbar . nbar (S.dd) per (row, head)
   for (int r = warp; r < TM; r += NT / 32) {
     for (int h = 0; h < H; ++h) {
@@ -511,9 +459,9 @@ __global__ void __launch_bounds__(NT, 1) pairs_bwd_kernel(EnfPairParams P) {
       float part[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
       for (int j = lane; j < HD; j += 32) {
         float dproj = Gv[r * C::LD + HD + j] * bufN[r * C::LD + j] - Gv[r * C::LD + j] * bufN[r * C::LD + HD + j];
-        for (int i = 0; i < P.I; ++i) part[i] = fmaf(dproj, S.omv[i * HD + j], part[i]);
+        for (int i = 0; i < P.rec.I; ++i) part[i] = fmaf(dproj, S.omv[i * HD + j], part[i]);
       }
-      for (int i = 0; i < P.I; ++i) {
+      for (int i = 0; i < P.rec.I; ++i) {
         float v = warp_sum(part[i]);
         if (lane == 0) S.du[r * 8 + i] = two_pi * v;
       }
@@ -544,9 +492,9 @@ __global__ void __launch_bounds__(NT, 1) pairs_bwd_kernel(EnfPairParams P) {
       float part[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
       for (int j = lane; j < HD; j += 32) {
         float dproj = Gq[r * C::LD + HD + j] * bufN[r * C::LD + j] - Gq[r * C::LD + j] * bufN[r * C::LD + HD + j];
-        for (int i = 0; i < P.I; ++i) part[i] = fmaf(dproj, S.omq[i * HD + j], part[i]);
+        for (int i = 0; i < P.rec.I; ++i) part[i] = fmaf(dproj, S.omq[i * HD + j], part[i]);
       }
-      for (int i = 0; i < P.I; ++i) {
+      for (int i = 0; i < P.rec.I; ++i) {
         float v = warp_sum(part[i]);
         if (lane == 0) S.du[r * 8 + i] += two_pi * v;
       }
@@ -555,59 +503,23 @@ __global__ void __launch_bounds__(NT, 1) pairs_bwd_kernel(EnfPairParams P) {
     // ---- invariants / window backward: cotangent of each record row, then reduce over the tile ----
     if (tid < TM) {
       const int t = tid;
-      float dq[ENF_R_LAM];
+      EnfPairRecord rec;
 #pragma unroll
-      for (int r = 0; r < ENF_R_LAM; ++r) dq[r] = 0.f;
+      for (int r = 0; r < 6; ++r) rec.u[r] = S.u[t * 8 + r];
+      rec.w = S.w[t]; rec.c = S.u[t * 8 + 7];
       float du[6];
-      for (int i = 0; i < 6; ++i) du[i] = i < P.I ? S.du[t * 8 + i] : 0.f;
+      for (int i = 0; i < 6; ++i) du[i] = i < P.rec.I ? S.du[t * 8 + i] : 0.f;
       float dw = 0.f;
       for (int h = 0; h < H; ++h) dw += S.aux[h * TM + t];
-      float dsg = 0.f;
-      if (P.win_kind != ENF_WIN_NONE) {
-        float sg = P.sigma[bz];
-        float inv_s2 = 1.f / (sg * sg);
-        float w = S.w[t];
-        if (P.win_kind == ENF_WIN_NP) {
-          dq[P.I] = -dw * inv_s2;
-          dsg = dw * (-2.f * w / sg);
-        } else if (P.win_kind == ENF_WIN_PER) {
-          du[0] += dw * 2.f * S.u[t * 8 + 0] * inv_s2;
-          du[1] += dw * 2.f * S.u[t * 8 + 1] * inv_s2;
-          dsg = dw * (-2.f * w / sg);
-        } else {
-          float c = S.u[t * 8 + 7];
-          float cl = fminf(fmaxf(c, -1.f + 1e-6f), 1.f - 1e-6f);
-          float ac = acosf(cl);
-          float dc = (c > -1.f + 1e-6f && c < 1.f - 1e-6f) ? dw * w * ac * inv_s2 * rsqrtf(1.f - cl * cl) : 0.f;
-          if (P.win_row >= 0) dq[P.I] = dc; else du[0] += dc;
-          dsg = dw * w * ac * ac * inv_s2 / sg;
-        }
-      }
-      for (int r = 0; r < P.I; ++r) {
-        if (P.row_kind == ENF_ROW_SQDIST_SQRT) {
-          float ur = S.u[t * 8 + r];
-          dq[r] = ur > 0.f ? du[r] / (2.f * ur) : 0.f;
-        } else {
-          dq[r] = du[r];
-        }
-      }
+      float dq[ENF_R_LAM], dsg;
+      record_adjoint(P.rec, rec, du, dw, P.sigma ? P.sigma[bz] : 1.f, dq, dsg);
 #pragma unroll
       for (int r = 0; r < ENF_R_LAM; ++r) S.dq[t * 8 + r] = dq[r];
       S.dsig[t] = dsg;
       if (P.g_xi) {
-        // cotangent of this row's QUERY record (self-attention: the queries are poses too, SURVEY 8f-4): DOT rows are bilinear
-        // in (Lam, xi); squared-distance rows (and the non-periodic window row) are sum_f (Lam_f - xi_f)^2
-        const int nrows = P.I + (P.win_row >= 0 ? 1 : 0);
-        for (int r = 0; r < nrows; ++r) {
-          const float* L = S.lam + r * ENF_F_XI;
-          const bool sq = r < P.I ? (P.row_kind != ENF_ROW_DOT) : (P.win_kind == ENF_WIN_NP);
-          if (sq) {
-            for (int f = 0; f < 3; ++f) if (f < P.nsq) gxi[f] = fmaf(-2.f * dq[r], L[f] - S.xi[t * 8 + f], gxi[f]);
-          } else {
-#pragma unroll
-            for (int f = 0; f < 8; ++f) gxi[f] = fmaf(dq[r], L[f], gxi[f]);
-          }
-        }
+        // cotangent of this row's QUERY record (self-attention: the queries are poses too, SURVEY 8f-4)
+        record_xi_cotangent(P.rec, S.lam, S.xi + t * 8, dq, 0, gxi);
+        record_xi_cotangent(P.rec, S.lam, S.xi + t * 8, dq, 1, gxi + 4);
       }
     }
     __syncthreads();
@@ -616,7 +528,7 @@ __global__ void __launch_bounds__(NT, 1) pairs_bwd_kernel(EnfPairParams P) {
       float v = 0.f;
       for (int t = 0; t < TM; ++t) v = fmaf(S.dq[t * 8 + r], S.xi[t * 8 + f], v);
       atomicAdd(P.g_lam + bz * ENF_LAM_SIZE + tid, v);
-    } else if (tid == 64 && P.win_kind != ENF_WIN_NONE) {
+    } else if (tid == 64 && P.rec.win_kind != ENF_WIN_NONE) {
       float v = 0.f;
       for (int t = 0; t < TM; ++t) v += S.dsig[t];
       atomicAdd(P.g_sigma + bz, v);

@@ -142,13 +142,12 @@ __global__ void __launch_bounds__(TcCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_fwd_tc
 #pragma unroll
     for (int k = 0; k < (6 + C::NQ - 1) / C::NQ; ++k) {
       const int i = cq + k * C::NQ;
-      if (i < P.I && i < 6) proj_store_pair(sU, i, row, inv_row(P, lat, xi_r, i), true);
+      if (i < P.rec.I && i < 6) proj_store_pair(sU, i, row, record_row(P.rec, lat, xi_r, i), true);
     }
     if (cq == C::NQ - 1) {
-      float u0 = 0.f, u1 = 0.f, w, c;
-      if (P.win_kind == ENF_WIN_PER) { u0 = inv_row(P, lat, xi_r, 0); u1 = inv_row(P, lat, xi_r, 1); }
-      else if (P.win_kind == ENF_WIN_SPH && P.win_row < 0) u0 = inv_row(P, lat, xi_r, 0);
-      window_value(P, lat, xi_r, P.sigma ? lat[64 + 2 * H * D + 4] : 1.f, u0, u1, w, c);
+      float u0, u1, w, c;
+      record_window_rows(P.rec, lat, xi_r, u0, u1);
+      record_window<true>(P.rec, lat, xi_r, P.sigma ? lat[64 + 2 * H * D + 4] : 1.f, u0, u1, w, c);
       s_win[wbuf * ROWS + row] = w;
     }
   };
@@ -175,8 +174,8 @@ __global__ void __launch_bounds__(TcCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_fwd_tc
   const uint32_t aU = tc::smem_u32(sU), aOm = tc::smem_u32(sOm);
 
   // Omega image [Omega_q | Omega_v]; invariants of latent 0; phases of latent 0
-  proj_build_omega(sOm, 0, P.q_omega, P.I, HD, tid, C::NT);
-  proj_build_omega(sOm, HD, P.v_omega, P.I, HD, tid, C::NT);
+  proj_build_omega(sOm, 0, P.q_omega, P.rec.I, HD, tid, C::NT);
+  proj_build_omega(sOm, HD, P.v_omega, P.rec.I, HD, tid, C::NT);
   __syncthreads();                             // latent 0's vectors are visible
   write_invariants(s_lat, 0);
   tc::fence_proxy_async();

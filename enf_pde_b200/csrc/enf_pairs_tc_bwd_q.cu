@@ -152,8 +152,8 @@ __global__ void __launch_bounds__(QCfg<D, H>::NTALL, D <= 64 ? 2 : 1) pairs_bwd_
                  aDz = tc::smem_u32(sDz), aS = tc::smem_u32(sS), aU = tc::smem_u32(sU), aOm = tc::smem_u32(sOm),
                  aOmT = tc::smem_u32(sOmT);
   // Omega images: projection operand (phases) and its transpose for du, both as a two-term fp16 split of 2 pi Omega
-  proj_build_omega(sOm, 0, P.q_omega, P.I, HD, tid, C::NTALL);
-  for (int e = tid; e < P.I * HD; e += C::NTALL) {
+  proj_build_omega(sOm, 0, P.q_omega, P.rec.I, HD, tid, C::NTALL);
+  for (int e = tid; e < P.rec.I * HD; e += C::NTALL) {
     const int i = e / HD, j = e % HD;
     const float val = 6.283185307179586f * P.q_omega[e];
     const __half hi = __float2half_rn(val);
@@ -189,8 +189,8 @@ __global__ void __launch_bounds__(QCfg<D, H>::NTALL, D <= 64 ? 2 : 1) pairs_bwd_
     };
     const uint32_t it0 = it;                           // row-record slot of tile ct of this item: (it0 + ct) % 3
     auto write_invariants = [&](int ct, const float* xi_r) {
-      const Rec rec = pair_record(P, s_lam, xi_r, sigma);
-      proj_write_u(sU, row, rec.u, P.I);
+      const EnfPairRecord rec = pair_record<true>(P.rec, s_lam, xi_r, sigma);
+      proj_write_u(sU, row, rec.u, P.rec.I);
       float4* rx = reinterpret_cast<float4*>(s_rx + (((it0 + ct) % 3) * ROWS + row) * C::RX);
       rx[0] = make_float4(xi_r[0], xi_r[1], xi_r[2], xi_r[3]);
       rx[1] = make_float4(xi_r[4], xi_r[5], xi_r[6], xi_r[7]);
@@ -215,7 +215,7 @@ __global__ void __launch_bounds__(QCfg<D, H>::NTALL, D <= 64 ? 2 : 1) pairs_bwd_
       const float4* rx = reinterpret_cast<const float4*>(s_rx + (((it0 + ct) % 3) * ROWS + row) * C::RX);
       const float4 x0 = rx[0], x1 = rx[1], r0 = rx[2], r1 = rx[3];
       const float xi_r[8] = {x0.x, x0.y, x0.z, x0.w, x1.x, x1.y, x1.z, x1.w};
-      Rec rec;
+      EnfPairRecord rec;
       rec.u[0] = r0.x; rec.u[1] = r0.y; rec.u[2] = r0.z; rec.u[3] = r0.w; rec.u[4] = r1.x; rec.u[5] = r1.y; rec.w = r1.z; rec.c = r1.w;
       const float dw = reinterpret_cast<const float*>(rx)[16];
       tc::mbar_wait(bar_u, par_u);
@@ -225,55 +225,14 @@ __global__ void __launch_bounds__(QCfg<D, H>::NTALL, D <= 64 ? 2 : 1) pairs_bwd_
       tc::tmem_ld_wait();
       float du[6];
 #pragma unroll
-      for (int i = 0; i < 6; ++i) du[i] = i < P.I ? d16[i] + d16[6 + i] + duv[i] : 0.f;
-      float dq[ENF_R_LAM];
-#pragma unroll
-      for (int r = 0; r < ENF_R_LAM; ++r) dq[r] = 0.f;
-      float dsg = 0.f;
-      if (P.win_kind != ENF_WIN_NONE) {
-        const float inv_s2 = 1.f / (sigma * sigma);
-        if (P.win_kind == ENF_WIN_NP) {
-          dq[P.I] = -dw * inv_s2;
-          dsg = dw * (-2.f * rec.w / sigma);
-        } else if (P.win_kind == ENF_WIN_PER) {
-          du[0] += dw * 2.f * rec.u[0] * inv_s2;
-          du[1] += dw * 2.f * rec.u[1] * inv_s2;
-          dsg = dw * (-2.f * rec.w / sigma);
-        } else {
-          float cl = fminf(fmaxf(rec.c, -1.f + 1e-6f), 1.f - 1e-6f);
-          float ac = acosf(cl);
-          float dc = (rec.c > -1.f + 1e-6f && rec.c < 1.f - 1e-6f) ? dw * rec.w * ac * inv_s2 * rsqrtf(1.f - cl * cl) : 0.f;
-          if (P.win_row >= 0) dq[P.I] = dc; else du[0] += dc;
-          dsg = dw * rec.w * ac * ac * inv_s2 / sigma;
-        }
-      }
-#pragma unroll
-      for (int r = 0; r < 6; ++r) {
-        if (r < P.I) {
-          if (P.row_kind == ENF_ROW_SQDIST_SQRT) dq[r] = rec.u[r] > 0.f ? du[r] / (2.f * rec.u[r]) : 0.f;
-          else dq[r] = du[r];
-        }
-      }
+      for (int i = 0; i < 6; ++i) du[i] = i < P.rec.I ? d16[i] + d16[6 + i] + duv[i] : 0.f;
+      float dq[ENF_R_LAM], dsg;
+      record_adjoint(P.rec, rec, du, dw, sigma, dq, dsg);
       if constexpr (GX) {
-        // d xi[f] for my half of the record (part 0: f = 0..3, part 1: f = 4..7): DOT rows are bilinear in (Lam, xi),
-        // squared-distance rows (and the non-periodic window row) are sum_{f < nsq} (Lam_f - xi_f)^2, nsq <= 3
+        // d xi[f] for my half of the record (part 0: f = 0..3, part 1: f = 4..7)
         if (ct * ROWS + row < P.C) {
-          const float* Lp = s_lam + 4 * part;
           float g[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll
-          for (int r = 0; r < ENF_R_LAM; ++r) {
-            if (r < P.I || (r == P.I && P.win_row >= 0)) {
-              const float* L = Lp + r * ENF_F_XI;
-              const bool sq = r < P.I ? (P.row_kind != ENF_ROW_DOT) : (P.win_kind == ENF_WIN_NP);
-              if (!sq) {
-#pragma unroll
-                for (int k = 0; k < 4; ++k) g[k] = fmaf(dq[r], L[k], g[k]);
-              } else if (part == 0) {
-#pragma unroll
-                for (int k = 0; k < 3; ++k) if (k < P.nsq) g[k] = fmaf(-2.f * dq[r], L[k] - xi_r[k], g[k]);
-              }
-            }
-          }
+          record_xi_cotangent(P.rec, s_lam, xi_r, dq, part, g);
           red_add_f32x4(P.g_xi + ((int64_t)b * P.C + ct * ROWS + row) * ENF_F_XI + 4 * part,
                         g[0] * inv_gs, g[1] * inv_gs, g[2] * inv_gs, g[3] * inv_gs);
         }
@@ -502,7 +461,7 @@ __global__ void __launch_bounds__(QCfg<D, H>::NTALL, D <= 64 ? 2 : 1) pairs_bwd_
     tc::tc_fence_before();
     __syncthreads();
     if (tid < ENF_LAM_SIZE) P.g_lam[bz * ENF_LAM_SIZE + tid] = s_dlam[tid] * inv_gs;
-    if (tid == ENF_LAM_SIZE && P.win_kind != ENF_WIN_NONE) P.g_sigma[bz] = s_dlam[ENF_LAM_SIZE] * inv_gs;
+    if (tid == ENF_LAM_SIZE && P.rec.win_kind != ENF_WIN_NONE) P.g_sigma[bz] = s_dlam[ENF_LAM_SIZE] * inv_gs;
     if (tid < H) P.g_kappa[bz * H + tid] = scale * inv_gs * s_dkap[tid];
   }
   // ---- CTA flush: shared-weight gradients --------------------------------------------------------------------------------

@@ -138,8 +138,8 @@ __global__ void __launch_bounds__(VCfg<D>::NT, D == 32 ? 2 : 1) pairs_bwd_tc_v_k
     *reinterpret_cast<__half*>(sOne + (k >> 6) * 2048 + ((((k & 63) >> 3) ^ 0) << 4) + (k & 7) * 2) = __float2half_rn(1.f);
   }
   // Omega images: projection operand (phases) and its transpose for du, both as a two-term fp16 split of 2 pi Omega
-  proj_build_omega(sOm, 0, P.v_omega, P.I, HD, tid, C::NT);
-  for (int e = tid; e < P.I * HD; e += C::NT) {
+  proj_build_omega(sOm, 0, P.v_omega, P.rec.I, HD, tid, C::NT);
+  for (int e = tid; e < P.rec.I * HD; e += C::NT) {
     const int i = e / HD, j = e % HD;
     const float val = 6.283185307179586f * P.v_omega[e];
     const __half hi = __float2half_rn(val);
@@ -172,8 +172,8 @@ __global__ void __launch_bounds__(VCfg<D>::NT, D == 32 ? 2 : 1) pairs_bwd_tc_v_k
       }
     };
     auto write_invariants = [&](const float* xi_r) {
-      const Rec rec = pair_record(P, s_lam, xi_r, sigma);
-      proj_write_u(sU, row, rec.u, P.I);
+      const EnfPairRecord rec = pair_record<true>(P.rec, s_lam, xi_r, sigma);
+      proj_write_u(sU, row, rec.u, P.rec.I);
     };
     // one thread per row: du of tile ct (value path) -> duv for kernel C
     auto store_du = [&](int ct, uint32_t par_u) {
@@ -185,7 +185,7 @@ __global__ void __launch_bounds__(VCfg<D>::NT, D == 32 ? 2 : 1) pairs_bwd_tc_v_k
       if (ct * ROWS + row < P.C) {
         float du[8];
 #pragma unroll
-        for (int i = 0; i < 8; ++i) du[i] = (i < 6 && i < P.I) ? d16[i] + d16[6 + i] : 0.f;
+        for (int i = 0; i < 8; ++i) du[i] = (i < 6 && i < P.rec.I) ? d16[i] + d16[6 + i] : 0.f;
         float4* dst = reinterpret_cast<float4*>(P.duv + (bz * P.C + ct * ROWS + row) * 8);
         dst[0] = make_float4(du[0], du[1], du[2], du[3]);
         dst[1] = make_float4(du[4], du[5], du[6], du[7]);

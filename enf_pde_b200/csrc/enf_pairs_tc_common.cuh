@@ -120,63 +120,6 @@ __device__ __forceinline__ float2 cos2_fma(float2 ph) {
                      __uint_as_float(__float_as_uint(p.y) ^ (__float_as_uint(t.y) << 31)));
 }
 
-struct Rec { float u[6]; float w; float c; };   // invariants, window value, raw cosine (spherical windows)
-
-// invariant row i of one (query, latent) pair: u_i = post(row_i(Lam, xi))
-template <class Params>
-__device__ __forceinline__ float inv_row(const Params& P, const float* lam, const float* x, int i) {
-  const float* L = lam + i * ENF_F_XI;
-  float v = 0.f;
-  if (P.row_kind == ENF_ROW_DOT) {
-#pragma unroll
-    for (int f = 0; f < 8; ++f) v = fmaf(L[f], x[f], v);
-  } else {
-#pragma unroll
-    for (int f = 0; f < 3; ++f) if (f < P.nsq) { float dl = L[f] - x[f]; v = fmaf(dl, dl, v); }
-    if (P.row_kind == ENF_ROW_SQDIST_SQRT) v = sqrtf(v);
-  }
-  return v;
-}
-// window value w (and the raw cosine c of the spherical windows) from the invariants it reads (u0, u1) and the window row
-template <class Params>
-__device__ __forceinline__ void window_value(const Params& P, const float* lam, const float* x, float sigma, float u0, float u1,
-                                             float& w, float& c) {
-  w = 0.f; c = 0.f;
-  if (P.win_kind == ENF_WIN_NONE) return;
-  const float* L = lam + P.I * ENF_F_XI;
-  float inv_s2 = 1.f / (sigma * sigma);
-  if (P.win_kind == ENF_WIN_NP) {
-    float v = 0.f;
-#pragma unroll
-    for (int f = 0; f < 3; ++f) if (f < P.nsq) { float dl = L[f] - x[f]; v = fmaf(dl, dl, v); }
-    w = -v * inv_s2;
-  } else if (P.win_kind == ENF_WIN_PER) {
-    w = (u0 * u0 + u1 * u1) * inv_s2;
-  } else {
-    c = u0;
-    if (P.win_row >= 0) {
-      c = 0.f;
-#pragma unroll
-      for (int f = 0; f < 8; ++f) c = fmaf(L[f], x[f], c);
-    }
-    float cl = fminf(fmaxf(c, -1.f + 1e-6f), 1.f - 1e-6f);
-    float ac = acosf(cl);
-    w = __expf(-ac * ac * 0.5f * inv_s2);
-  }
-}
-
-template <class Params>
-__device__ __forceinline__ Rec pair_record(const Params& P, const float* lam, const float* xi, float sigma) {
-  Rec r;
-  float x[8];
-#pragma unroll
-  for (int f = 0; f < 8; ++f) x[f] = xi[f];
-#pragma unroll
-  for (int i = 0; i < 6; ++i) r.u[i] = i < P.I ? inv_row(P, lam, x, i) : 0.f;
-  window_value(P, lam, x, sigma, r.u[0], r.u[1], r.w, r.c);
-  return r;
-}
-
 // gamma(u) = [sin(2 pi u Omega) | cos(2 pi u Omega)] (rff.py:84-93)
 // ---- RFF projection on the tensor core ---------------------------------------------------------------------------
 // proj[row][n] = 2 pi sum_i u[row][i] Omega[i][n] as ONE small MMA per 128-row tile (M = 128, N = #frequencies, K = 32)

@@ -792,14 +792,14 @@ int enf_launch_pose_record_bwd(cudaStream_t st, int kind, int Dx, int P, int I, 
 }
 
 int enf_launch_latent_record(cudaStream_t st, const EnfDesc& d, const float* p, float* lam) {
-  EnfRecordLayout r = enf_record_layout(d.invariant_kind, d.Dx, d.use_window);
+  EnfInvariantLayout r = enf_record_layout(d.invariant_kind, d.Dx, d.use_window);
   int64_t total = (int64_t)d.B * d.Z;
   latent_record_kernel<<<blocks_for(total, 128), 128, 0, st>>>(d.invariant_kind, d.Dx, r.P, r.I, total, p, lam, 0);
   return 1;
 }
 
 int enf_launch_latent_record_bwd(cudaStream_t st, const EnfDesc& d, const float* p, const float* dlam, float* dp) {
-  EnfRecordLayout r = enf_record_layout(d.invariant_kind, d.Dx, d.use_window);
+  EnfInvariantLayout r = enf_record_layout(d.invariant_kind, d.Dx, d.use_window);
   int64_t total = (int64_t)d.B * d.Z;
   latent_record_bwd_kernel<<<blocks_for(total, 128), 128, 0, st>>>(d.invariant_kind, d.Dx, r.P, r.I, r.win_kind, total,
                                                                    p, dlam, dp, 0);
