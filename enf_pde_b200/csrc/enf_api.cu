@@ -110,7 +110,8 @@ int validate(const EnfDesc* D, EnfInvariantLayout* rl) {
   return ENF_OK;
 }
 
-// tensor-core backward wherever the tensor-core forward runs (d in {64, 128}, H <= 2): a backward on the fp32 kernels behind a
+// tensor-core backward wherever the tensor-core forward runs (d in {32, 64, 128}, H <= 4; more than two heads at d >= 64, and
+// four at d = 32, run as head groups of <= 2): a backward on the fp32 kernels behind a
 // 16-bit-operand forward mixes two different roundings of the same activations (measured: 2e-2 on single weight-gradient leaves)
 bool use_tc_bwd(const EnfDesc& D) { return tc_fwd_on(D) && enf_pairs_bwd_tc_supported(D.d, D.H); }
 

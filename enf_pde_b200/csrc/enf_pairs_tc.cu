@@ -54,16 +54,19 @@ template <int D, int H> struct TcCfg {
   // per-latent vectors are double buffered (cp.async prefetch of the next latent): [2] x { Lam 64 | U H*D | b3 H*D | kappa, sigma 8 }
   static constexpr int F_LAT = 64 + 2 * H * D + 8;
   static constexpr int F_WIN = 2 * ROWS, F_BIAS = 3 * D, F_EXCH = NQ * ROWS * 2 + NQ * ROWS * (H > 2 ? H : 2);
-  static_assert(H <= 2 || D == 32, "three heads: num_hidden = 32 only (TMEM: T0 | T1 | H accumulators | phases)");
+  static_assert(H <= 2 || D == 32, "three heads in one kernel: num_hidden = 32 only (TMEM: T0 | T1 | H accumulators | phases); more run as head groups");
   static_assert(H <= 3, "the logit partials [NQ][ROWS][H] share exchange buffer 1");
   static constexpr int F_TOTAL = 2 * F_LAT + F_WIN + F_BIAS + F_EXCH;
   static constexpr uint32_t SMEM_BYTES = OFF_F + F_TOTAL * 4 + 128 /*barriers*/ + 1024 /*alignment slack*/;
   static_assert(SMEM_BYTES <= 227 * 1024, "shared memory budget");
 };
 
-template <int D, int H>
-__global__ void __launch_bounds__(TcCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_fwd_tc_kernel(EnfPairTcParams P) {
+// G (head group): the kernel runs heads h0 .. h0 + H - 1 of a description with HT heads in all (one launch per group, see
+// enf_launch_pairs_fwd_tc); every per-head tensor keeps its full-HT layout.  G = false: HT = H, h0 = 0, the arguments are unused.
+template <int D, int H, bool G>
+__global__ void __launch_bounds__(TcCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_fwd_tc_kernel(EnfPairTcParams P, int h0_arg, int HT_arg) {
   using C = TcCfg<D, H>;
+  const int HT = G ? HT_arg : H, h0 = G ? h0_arg : 0;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* base = smem_raw + ((1024u - (tc::smem_u32(smem_raw) & 1023u)) & 1023u);   // 1024-aligned; pointer stays in the shared address space (LDS/STS, not generic LD/ST)
   uint8_t* sW = base + C::OFF_W;
@@ -109,13 +112,14 @@ __global__ void __launch_bounds__(TcCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_fwd_tc
     const int64_t q = (int64_t)b * P.Z + z;
     float* dst = s_lat + (z & 1) * C::F_LAT;
     constexpr int NU = H * D / 4;
-    if (tid < NU) tc::cp_async<16>(dst + 64 + 4 * tid, P.U + q * H * D + 4 * tid);
-    else if (tid < 2 * NU) tc::cp_async<16>(dst + 64 + H * D + 4 * (tid - NU), P.b3 + q * H * D + 4 * (tid - NU));
+    const int64_t qh = G ? q * HT + h0 : q * H;        // this group's first head of latent q
+    if (tid < NU) tc::cp_async<16>(dst + 64 + 4 * tid, P.U + qh * D + 4 * tid);
+    else if (tid < 2 * NU) tc::cp_async<16>(dst + 64 + H * D + 4 * (tid - NU), P.b3 + qh * D + 4 * (tid - NU));
     else if (tid < 2 * NU + ENF_LAM_SIZE / 4) tc::cp_async<16>(dst + 4 * (tid - 2 * NU), P.lam + q * ENF_LAM_SIZE + 4 * (tid - 2 * NU));
     else if (tid == 2 * NU + ENF_LAM_SIZE / 4) {
-      if (H == 3) {          // 12 bytes is not a cp.async size (and q * 12 bytes is only 4-byte aligned)
+      if (H == 3 || G) {     // 12 bytes is not a cp.async size (and q * 12 bytes, or a group at an odd head, is only 4-byte aligned)
 #pragma unroll
-        for (int h = 0; h < H; ++h) tc::cp_async<4>(dst + 64 + 2 * H * D + h, P.kappa + q * H + h);
+        for (int h = 0; h < H; ++h) tc::cp_async<4>(dst + 64 + 2 * H * D + h, P.kappa + qh + h);
       } else {
         tc::cp_async<4 * (H == 3 ? 1 : H)>(dst + 64 + 2 * H * D, P.kappa + q * H);
       }
@@ -168,7 +172,7 @@ __global__ void __launch_bounds__(TcCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_fwd_tc
     tc::bulk_g2s(sW + C::WIMG, P.img_v_w1, C::WIMG, bar_w);
     tc::bulk_g2s(sW + 2 * C::WIMG, P.img_Wp, C::WIMG, bar_w);
     tc::mbar_expect_tx(&bar_w3[0], C::SBYTES);
-    tc::bulk_g2s(sS, P.img_W3 + ((int64_t)b * P.Z * H) * C::WIMG, C::SBYTES, &bar_w3[0]);
+    tc::bulk_g2s(sS, P.img_W3 + ((int64_t)b * P.Z * HT + h0) * C::WIMG, C::SBYTES, &bar_w3[0]);
   }
   const uint32_t aA0 = tc::smem_u32(sA0), aA1 = tc::smem_u32(sA1), aS = tc::smem_u32(sS), aW = tc::smem_u32(sW);
   const uint32_t aU = tc::smem_u32(sU), aOm = tc::smem_u32(sOm);
@@ -298,7 +302,7 @@ __global__ void __launch_bounds__(TcCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_fwd_tc
 #pragma unroll
       for (int q = 0; q < C::NQ; ++q) dot += s_spart[(q * ROWS + row) * H + h];
       float sv = scale * (dot + s_kap[h]) + win;
-      if (cq == 0 && row_valid && P.slog) P.slog[((bz * P.C) + c0 + row) * H + h] = sv;
+      if (cq == 0 && row_valid && P.slog) P.slog[((bz * P.C) + c0 + row) * HT + h0 + h] = sv;
       float m_new = fmaxf(m_run[h], sv);
       corr[h] = __expf(m_run[h] - m_new);
       pw[h] = __expf(sv - m_new);
@@ -311,7 +315,7 @@ __global__ void __launch_bounds__(TcCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_fwd_tc
     tc::tc_fence_after();
     if (H > 1 && !C::kStageAll && tid == 0) {          // A0 is free again: stream W3[z,1] into it
       tc::mbar_expect_tx(&bar_w3[1], C::WIMG);
-      tc::bulk_g2s(sA0, P.img_W3 + (bz * H + 1) * C::WIMG, C::WIMG, &bar_w3[1]);
+      tc::bulk_g2s(sA0, P.img_W3 + (bz * HT + h0 + 1) * C::WIMG, C::WIMG, &bar_w3[1]);
     }
     tc::tmem_ld32(t0 + my_t, v);
     tc::tmem_ld_wait();
@@ -418,7 +422,7 @@ __global__ void __launch_bounds__(TcCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_fwd_tc
       if (P.that_img) tc::bulk_wait_read0();   // the stashes have been read out of A1 / the stage buffer before they are overwritten
       if (more) {                              // stage buffer: next latent's W3[.,0] (needed by its GEMM4_0, most of a latent away)
         tc::mbar_expect_tx(&bar_w3[0], C::SBYTES);
-        tc::bulk_g2s(sS, P.img_W3 + ((bz + 1) * H) * C::WIMG, C::SBYTES, &bar_w3[0]);
+        tc::bulk_g2s(sS, P.img_W3 + ((bz + 1) * HT + h0) * C::WIMG, C::SBYTES, &bar_w3[0]);
       }
     }
     tc::tmem_st_wait();
@@ -433,11 +437,11 @@ __global__ void __launch_bounds__(TcCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_fwd_tc
     tc::tmem_ld_wait();
     if (row_valid) {
       float inv_l = 1.f / l_run[h];
-      float* o = P.nbar + (((int64_t)b * P.C + c0 + row) * H + h) * D + col0;
+      float* o = P.nbar + (((int64_t)b * P.C + c0 + row) * HT + h0 + h) * D + col0;
 #pragma unroll
       for (int j = 0; j < 32; j += 4)
         *reinterpret_cast<float4*>(o + j) = make_float4(a[j] * inv_l, a[j + 1] * inv_l, a[j + 2] * inv_l, a[j + 3] * inv_l);
-      if (cq == 0) P.lse[((int64_t)b * P.C + c0 + row) * H + h] = m_run[h] + logf(l_run[h]);
+      if (cq == 0) P.lse[((int64_t)b * P.C + c0 + row) * HT + h0 + h] = m_run[h] + logf(l_run[h]);
     }
   }
   tc::tc_fence_before();
@@ -445,21 +449,40 @@ __global__ void __launch_bounds__(TcCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_fwd_tc
   if (warp == 0) tc::tmem_dealloc<C::TMEM_COLS>(tm);
 }
 
-template <int D, int H>
-int launch_tc(cudaStream_t st, const EnfPairTcParams& p) {
+template <int D, int H, bool G = false>
+int launch_tc(cudaStream_t st, const EnfPairTcParams& p, int h0 = 0, int HT = H) {
   using C = TcCfg<D, H>;
-  if (cudaFuncSetAttribute(pairs_fwd_tc_kernel<D, H>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES) != cudaSuccess)
+  if (cudaFuncSetAttribute(pairs_fwd_tc_kernel<D, H, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM_BYTES) != cudaSuccess)
     return -1;
   dim3 grid((p.C + ROWS - 1) / ROWS, p.B);
-  pairs_fwd_tc_kernel<D, H><<<grid, C::NT, C::SMEM_BYTES, st>>>(p);
+  pairs_fwd_tc_kernel<D, H, G><<<grid, C::NT, C::SMEM_BYTES, st>>>(p, h0, HT);
   return 1;
+}
+
+// More heads than one kernel holds in TMEM: one launch per group of at most two heads (H = 3: 2 + 1, H = 4: 2 + 2).  Every
+// launch recomputes the shared value and query path; only the first writes the backward's stash, which does not depend on
+// the heads.
+template <int D>
+int launch_tc_groups(cudaStream_t st, int H, const EnfPairTcParams& p) {
+  EnfPairTcParams q = p;
+  int n = 0;
+  for (int h0 = 0; h0 < H; h0 += 2) {
+    const int r = H - h0 >= 2 ? launch_tc<D, 2, true>(st, q, h0, H) : launch_tc<D, 1, true>(st, q, h0, H);
+    if (r < 0) return -1;
+    n += r;
+    q.that_img = nullptr; q.dgr = nullptr; q.trstd = nullptr;
+  }
+  return n;
 }
 
 }  // namespace
 
-bool enf_pairs_fwd_tc_supported(int d, int H) { return ((d == 128 || d == 64) && (H == 1 || H == 2)) || (d == 32 && H >= 1 && H <= 3); }
+bool enf_pairs_fwd_tc_supported(int d, int H) { return (d == 128 || d == 64 || d == 32) && H >= 1 && H <= 4; }
 
 int enf_launch_pairs_fwd_tc(cudaStream_t st, int d, int H, const EnfPairTcParams& p) {
+  if (d == 32 && H == 4) return launch_tc_groups<32>(st, H, p);
+  if (d == 128 && H > 2) return launch_tc_groups<128>(st, H, p);
+  if (d == 64 && H > 2) return launch_tc_groups<64>(st, H, p);
   if (d == 32 && H == 3) return launch_tc<32, 3>(st, p);
   if (d == 32 && H == 2) return launch_tc<32, 2>(st, p);
   if (d == 32 && H == 1) return launch_tc<32, 1>(st, p);

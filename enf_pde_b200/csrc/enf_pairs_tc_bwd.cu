@@ -30,7 +30,7 @@ template <int D, int H> struct BwdCfg {
   static constexpr uint32_t ABLK = ROWS * 128;
   static constexpr uint32_t ATILE = atile_bytes<D>();
   static constexpr int HD = D / 2;
-  static_assert(H <= 2 || D == 32, "three heads: num_hidden = 32 only");
+  static_assert(H <= 2 || D == 32, "three heads in one kernel A: num_hidden = 32 only; more run as head groups");
 };
 
 __device__ __forceinline__ void load_scale(const float* gmax, float& gs, float& inv_gs) {
@@ -129,10 +129,15 @@ using tc::named_arrive;
 using tc::named_sync;
 
 // Warp 0 issues (bulk copies, tcgen05.mma, commits) between its own epilogue phases.
-template <int D, int H>
-__global__ void __launch_bounds__(BwdCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_bwd_tc_a_kernel(EnfPairTcBwdParams P) {
+// G (head group): the kernel runs heads h0 .. h0 + H - 1 of a description with HT heads in all (one launch per group, see
+// launch_main_groups); every per-head tensor keeps its full-HT layout.  dthat = sum over ALL heads: a group with h0 > 0 adds its
+// part to the one the previous groups stored (fp32 add of the stored fp16 value, then one more rounding).  G = false: HT = H,
+// h0 = 0, the arguments are unused.
+template <int D, int H, bool G>
+__global__ void __launch_bounds__(BwdCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_bwd_tc_a_kernel(EnfPairTcBwdParams P, int h0_arg, int HT_arg) {
   using C = BwdCfg<D, H>;
   using A = ACfg<D, H>;
+  const int HT = G ? HT_arg : H, h0 = G ? h0_arg : 0;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* base = smem_raw + ((1024u - (tc::smem_u32(smem_raw) & 1023u)) & 1023u);   // 1024-aligned; pointer stays in the shared address space (LDS/STS, not generic LD/ST)
   uint8_t* sW3 = base + A::OFF_W3;
@@ -166,7 +171,7 @@ __global__ void __launch_bounds__(BwdCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_bwd_t
   constexpr int kTmemNeed = (kWork + H) * D;
   constexpr int kTmemCols = kTmemNeed <= 128 ? 128 : kTmemNeed <= 256 ? 256 : 512;
   if (warp == 0) tc::tmem_alloc<kTmemCols>(s_tmem);
-  for (int e = tid; e < H * D; e += C::NT) { s_b3[e] = P.b3[bz * H * D + e]; s_db3[e] = 0.f; }
+  for (int e = tid; e < H * D; e += C::NT) { s_b3[e] = P.b3[(G ? (bz * HT + h0) * D : bz * H * D) + e]; s_db3[e] = 0.f; }
   float gs, inv_gs;
   load_scale(P.gmax, gs, inv_gs);
   tc::tc_fence_before();
@@ -181,7 +186,7 @@ __global__ void __launch_bounds__(BwdCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_bwd_t
   // ---- what the issuing lane does at the three issue points of a tile ------------------------------------------------------
   auto issue_prologue = [&]() {
     tc::mbar_expect_tx(bar_w, H * C::WIMG);
-    for (int h = 0; h < H; ++h) tc::bulk_g2s(sW3 + h * C::WIMG, P.img_W3 + (bz * H + h) * C::WIMG, C::WIMG, bar_w);
+    for (int h = 0; h < H; ++h) tc::bulk_g2s(sW3 + h * C::WIMG, P.img_W3 + (G ? bz * HT + h0 + h : bz * H + h) * C::WIMG, C::WIMG, bar_w);
     tc::mbar_expect_tx(&bar_t[0], C::ATILE);
     tc::bulk_g2s(sT, timg, C::ATILE, &bar_t[0]);
     tc::mbar_wait(bar_w, 0);
@@ -237,12 +242,12 @@ __global__ void __launch_bounds__(BwdCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_bwd_t
     if (cq == 0 && c < P.C) {
       const int64_t q = (int64_t)b * P.C + c;
       float* dst = s_rs + (ct & 1) * 3 * ROWS * H + row * H;
-      if (H == 3) {        // 12 bytes is not a cp.async size
+      if (H == 3 || G) {   // 12 bytes is not a cp.async size; a group of two at an odd head (or of HT = 3) is only 4-byte aligned
 #pragma unroll
         for (int h = 0; h < H; ++h) {
-          tc::cp_async<4>(dst + h, P.slog + (bz * P.C + c) * H + h);
-          tc::cp_async<4>(dst + ROWS * H + h, P.lse + q * H + h);
-          tc::cp_async<4>(dst + 2 * ROWS * H + h, P.Dg + q * H + h);
+          tc::cp_async<4>(dst + h, P.slog + (bz * P.C + c) * HT + h0 + h);
+          tc::cp_async<4>(dst + ROWS * H + h, P.lse + q * HT + h0 + h);
+          tc::cp_async<4>(dst + 2 * ROWS * H + h, P.Dg + q * HT + h0 + h);
         }
       } else {
         constexpr int kB = 4 * (H == 3 ? 1 : H);
@@ -259,7 +264,7 @@ __global__ void __launch_bounds__(BwdCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_bwd_t
   prefetch_rows(0);
   uint4 dnq[4];                                      // my 32 columns of the scaled fp16 cotangent of nbar, (tile, head) about to be processed
   auto load_dnb = [&](int ct, int h) {
-    const uint4* src = P.dnb16 + ((((int64_t)b * ntiles + ct) * H + h) * C::NQ + cq) * 4 * ROWS + row;
+    const uint4* src = P.dnb16 + ((((int64_t)b * ntiles + ct) * HT + h0 + h) * C::NQ + cq) * 4 * ROWS + row;
 #pragma unroll
     for (int q = 0; q < 4; ++q) dnq[q] = __ldg(src + q * ROWS);       // a warp reads 512 contiguous bytes per instruction
   };
@@ -358,7 +363,7 @@ __global__ void __launch_bounds__(BwdCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_bwd_t
         float cs = warp_colsum32_h2(dmh, lane);
         atomicAdd(&s_db3[h * D + col0 + lane], cs);
       }
-      if (cq == 0 && valid) P.ds[((bz * P.C) + c0 + row) * H + h] = dsh;
+      if (cq == 0 && valid) P.ds[((bz * P.C) + c0 + row) * HT + h0 + h] = dsh;
     }
     // dthat = sum_h dm_h W3_h^T -> global (fp16, scaled)
     tc::mbar_wait(bar_d, par);
@@ -369,6 +374,17 @@ __global__ void __launch_bounds__(BwdCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_bwd_t
     if (ct + 1 < ntiles && warp != 0) named_arrive(kABarDth, C::NT);     // tF may be overwritten by the next tile's second G4
     {                                                // chunked order: a warp stores 512 contiguous bytes per instruction
       uint4* dst = reinterpret_cast<uint4*>(P.dthat) + ((bz * ntiles + ct) * C::NQ + cq) * 4 * ROWS + row;
+      if constexpr (G) {
+        if (h0 > 0) {                                // the earlier groups' part of dthat
+#pragma unroll
+          for (int q = 0; q < 4; ++q) {
+            const uint4 prev = dst[q * ROWS];
+            const __half2* p2 = reinterpret_cast<const __half2*>(&prev);
+#pragma unroll
+            for (int t = 0; t < 4; ++t) tc::st2(v + q * 8 + 2 * t, tc::add2(tc::ld2(v + q * 8 + 2 * t), __half22float2(p2[t])));
+          }
+        }
+      }
 #pragma unroll
       for (int q = 0; q < 4; ++q) {
         uint4 u;
@@ -392,20 +408,20 @@ __global__ void __launch_bounds__(BwdCfg<D, H>::NT, D <= 64 ? 2 : 1) pairs_bwd_t
     tc::tmem_ld32(tW3 + h * D + my_t, w);
     tc::tmem_ld_wait();
     if (wrow >= 0) {
-      float* o = P.g_W3 + ((bz * H + h) * D + wrow) * D + col0;
+      float* o = P.g_W3 + ((G ? bz * HT + h0 + h : bz * H + h) * D + wrow) * D + col0;
 #pragma unroll
       for (int j = 0; j < 32; j += 4)
         *reinterpret_cast<float4*>(o + j) = make_float4(w[j] * inv_gs, w[j + 1] * inv_gs, w[j + 2] * inv_gs, w[j + 3] * inv_gs);
     }
   }
-  for (int e = tid; e < H * D; e += C::NT) P.g_b3[bz * H * D + e] = s_db3[e] * inv_gs;
+  for (int e = tid; e < H * D; e += C::NT) P.g_b3[(G ? (bz * HT + h0) * D : bz * H * D) + e] = s_db3[e] * inv_gs;
   tc::tc_fence_before();
   __syncthreads();
   if (warp == 0) tc::tmem_dealloc<kTmemCols>(tm);
 }
 
-template <int D, int H>
-int launch_prep(cudaStream_t st, const EnfPairTcBwdParams& p) {
+template <int D>
+int launch_prep(cudaStream_t st, int H, const EnfPairTcBwdParams& p) {
   const int64_t n4 = (int64_t)p.B * p.C * H * D / 4;
   int blocks = (int)((n4 + 255) / 256);
   if (blocks > 148 * 8) blocks = 148 * 8;
@@ -415,34 +431,53 @@ int launch_prep(cudaStream_t st, const EnfPairTcBwdParams& p) {
   return 2;
 }
 
-template <int D, int H>
-int launch_main(cudaStream_t st, const EnfPairTcBwdParams& p) {
+template <int D, int H, bool G = false>
+int launch_a(cudaStream_t st, const EnfPairTcBwdParams& p, int h0 = 0, int HT = H) {
   using C = BwdCfg<D, H>;
   size_t smem_a = ACfg<D, H>::SMEM_BYTES;
-  if (cudaFuncSetAttribute(pairs_bwd_tc_a_kernel<D, H>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_a) != cudaSuccess) return -1;
+  if (cudaFuncSetAttribute(pairs_bwd_tc_a_kernel<D, H, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_a) != cudaSuccess) return -1;
   const unsigned grid = (unsigned)(p.B * p.Z);
-  pairs_bwd_tc_a_kernel<D, H><<<grid, C::NT, smem_a, st>>>(p);
+  pairs_bwd_tc_a_kernel<D, H, G><<<grid, C::NT, smem_a, st>>>(p, h0, HT);
+  return 1;
+}
+
+template <int D, int H>
+int launch_main(cudaStream_t st, const EnfPairTcBwdParams& p) {
+  if (launch_a<D, H>(st, p) < 0) return -1;
   if (enf_launch_pairs_bwd_tc_v(st, D, p) < 0) return -1;
   if (enf_launch_pairs_bwd_tc_q(st, D, H, p) < 0) return -1;
   return 3;
 }
 
+// More heads than kernel A holds in TMEM: one kernel A per group of at most two heads (H = 3: 2 + 1, H = 4: 2 + 2), in head
+// order, the later groups adding to dthat; kernel B does not depend on the heads and kernel C runs once with all of them.
+template <int D>
+int launch_main_groups(cudaStream_t st, int H, const EnfPairTcBwdParams& p) {
+  int n = 0;
+  for (int h0 = 0; h0 < H; h0 += 2) {
+    if ((H - h0 >= 2 ? launch_a<D, 2, true>(st, p, h0, H) : launch_a<D, 1, true>(st, p, h0, H)) < 0) return -1;
+    ++n;
+  }
+  if (enf_launch_pairs_bwd_tc_v(st, D, p) < 0) return -1;
+  if (enf_launch_pairs_bwd_tc_q(st, D, H, p) < 0) return -1;
+  return n + 2;
+}
+
 }  // namespace
 
-bool enf_pairs_bwd_tc_supported(int d, int H) { return ((d == 128 || d == 64) && (H == 1 || H == 2)) || (d == 32 && H >= 1 && H <= 3); }
+bool enf_pairs_bwd_tc_supported(int d, int H) { return (d == 128 || d == 64 || d == 32) && H >= 1 && H <= 4; }
 
 int enf_launch_pairs_bwd_tc_prep(cudaStream_t st, int d, int H, const EnfPairTcBwdParams& p) {
-  if (d == 32 && H == 3) return launch_prep<32, 3>(st, p);
-  if (d == 32 && H == 2) return launch_prep<32, 2>(st, p);
-  if (d == 32 && H == 1) return launch_prep<32, 1>(st, p);
-  if (d == 128 && H == 2) return launch_prep<128, 2>(st, p);
-  if (d == 128 && H == 1) return launch_prep<128, 1>(st, p);
-  if (d == 64 && H == 2) return launch_prep<64, 2>(st, p);
-  if (d == 64 && H == 1) return launch_prep<64, 1>(st, p);
-  return -1;
+  if (!enf_pairs_bwd_tc_supported(d, H)) return -1;
+  if (d == 32) return launch_prep<32>(st, H, p);
+  if (d == 128) return launch_prep<128>(st, H, p);
+  return launch_prep<64>(st, H, p);
 }
 
 int enf_launch_pairs_bwd_tc_main(cudaStream_t st, int d, int H, const EnfPairTcBwdParams& p) {
+  if (d == 32 && H == 4) return launch_main_groups<32>(st, H, p);
+  if (d == 128 && H > 2) return launch_main_groups<128>(st, H, p);
+  if (d == 64 && H > 2) return launch_main_groups<64>(st, H, p);
   if (d == 32 && H == 3) return launch_main<32, 3>(st, p);
   if (d == 32 && H == 2) return launch_main<32, 2>(st, p);
   if (d == 32 && H == 1) return launch_main<32, 1>(st, p);

@@ -35,7 +35,9 @@ template <int D, int H> struct QCfg {
   static constexpr int NTALL = NT + NSIDE;
   static constexpr int TMEM_NEED = 2 * D + 64 + 48;           // T | dW1_q | phases (64) | db1q | dU | du (16 each)
   static constexpr int TMEM_COLS = TMEM_NEED <= 256 ? 256 : 512;
-  static_assert(1 + 2 * H <= 8, "side operand row: [1 | ds_hi (H) | ds_lo (H)] in 8 halves");
+  // side operand row [1 | ds_hi (H) | ds_lo (H)]: one 16-byte chunk (8 halves) up to H = 3, both chunks the N = 16 MMAs read at H = 4
+  static constexpr int NSIDE_HALVES = 1 + 2 * H <= 8 ? 8 : 16;
+  static_assert(1 + 2 * H <= 16, "side operand row: [1 | ds_hi (H) | ds_lo (H)] in 16 halves");
   static constexpr uint32_t OFF_W = 0;                         // W1_q image, W1_q low image
   static constexpr uint32_t OFF_GHI = 2 * WIMG;                // gamma_q hi
   static constexpr uint32_t OFF_GLO = OFF_GHI + ATILE;         // gamma_q lo -> h1q -> dproj
@@ -305,16 +307,18 @@ __global__ void __launch_bounds__(QCfg<D, H>::NTALL, D <= 64 ? 2 : 1) pairs_bwd_
       // ---- per-row side work, overlapped with the 3-term GEMM: shared by three of the row's four threads ----------------
       if (cq == 0) {
         {                                                  // side operand row: [1 | ds_hi | ds_lo | 0 ...]
-          __half hv[8];
+          __half hv[C::NSIDE_HALVES];
           hv[0] = __float2half_rn(1.f);
 #pragma unroll
-          for (int k = 1; k < 8; ++k) hv[k] = __float2half_rn(0.f);
+          for (int k = 1; k < C::NSIDE_HALVES; ++k) hv[k] = __float2half_rn(0.f);
 #pragma unroll
           for (int h = 0; h < H; ++h) {
             hv[1 + h] = __float2half_rn(dsv[h]);
             hv[1 + H + h] = __float2half_rn(dsv[h] - __half2float(hv[1 + h]));
           }
-          *reinterpret_cast<uint4*>(sS + tc::swz_chunk_off(row, 0)) = *reinterpret_cast<const uint4*>(hv);
+#pragma unroll
+          for (int k = 0; k < C::NSIDE_HALVES / 8; ++k)
+            *reinterpret_cast<uint4*>(sS + tc::swz_chunk_off(row, k)) = *reinterpret_cast<const uint4*>(hv + 8 * k);
         }
         float dw = 0.f;
 #pragma unroll
@@ -509,6 +513,11 @@ int launch_q(cudaStream_t st, const EnfPairTcBwdParams& p) { return p.g_xi ? lau
 }  // namespace
 
 int enf_launch_pairs_bwd_tc_q(cudaStream_t st, int d, int H, const EnfPairTcBwdParams& p) {
+  if (d == 32 && H == 4) return launch_q<32, 4>(st, p);
+  if (d == 128 && H == 4) return launch_q<128, 4>(st, p);
+  if (d == 128 && H == 3) return launch_q<128, 3>(st, p);
+  if (d == 64 && H == 4) return launch_q<64, 4>(st, p);
+  if (d == 64 && H == 3) return launch_q<64, 3>(st, p);
   if (d == 32 && H == 3) return launch_q<32, 3>(st, p);
   if (d == 32 && H == 2) return launch_q<32, 2>(st, p);
   if (d == 32 && H == 1) return launch_q<32, 1>(st, p);

@@ -50,7 +50,10 @@ enum EnfInvariantKind {
 
 enum EnfPrecision {
   ENF_PREC_FP32 = 0,   /* fp32 FMA everywhere: the <= 1e-4 parity bucket                       */
-  ENF_PREC_BF16 = 1    /* tcgen05 tensor cores, 16-bit operands, fp32 accumulate: <= 2e-3 bucket */
+  ENF_PREC_BF16 = 1    /* tcgen05 tensor cores, 16-bit operands, fp32 accumulate: <= 2e-3 bucket.  Pair kernels on the tensor
+                          cores for num_hidden 32, 64, 128 and every num_heads 1..4 (beyond two heads at 64 / 128, and
+                          four at 32, the forward and backward kernel A run once per group of <= 2 heads); num_hidden 16
+                          runs the fp32 pair kernels.  enf_xattn_dispatch reports which. */
 };
 
 /* EnfDesc.flags */
